@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- overlap-graph build throughput (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 3] [--scale 1.0]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 3] [--scale 1.0] [--dump-outputs DIR]
 
 Workload: BASELINE.json configs[2] (config 3: 20-genome mock metagenome, 10 M x 100 bp reads, minOverlap 50) -- the
 largest configuration one GPU holds; N GPUs build config 3 at N times the genomes and reads (weak scaling, N x 10 M reads).
@@ -21,12 +21,19 @@ the unmodified reference) on a bounded sample.
 
 --impl reference runs that CPU implementation as the measured arm (rank 0 only; this arm never imports the package or
 maps libogb.so: the sample is generated with numpy and the reference runs as a subprocess).
+
+--dump-outputs DIR writes what the last timed step computed, as a caller of the build receives it, to DIR/<name>.npy (rank 0,
+float64, < 64 MB in all): edges.npy (k, 4) [src, dst, offset, orient] rows of the final edge list in its canonical order (all
+rows, or a seeded sample of 2^20 row positions in ascending order), super_read_ids.npy (superReadID of reads 1..n, or a seeded
+sample of 2^21 of them), edge_checksum.npy (the device's order-independent [xor, sum] over every final edge, each 64-bit word
+as four 16-bit limbs, low first) and counts.npy [unique reads, pre-reduction edges, final edges, nodes, contained reads].
+The inputs are seeded: the same arguments give the same inputs on every run, so two builds can be compared file by file.
+The bench reads the tree as __graft_entry__.build() left it and writes nothing there.
 """
 import argparse
 import ctypes as C
 import json
 import os
-import subprocess
 import sys
 import tempfile
 import threading
@@ -34,6 +41,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True        # the tree may be read-only: no __pycache__ next to the modules imported below
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -208,8 +216,6 @@ def cpu_reference(cfg_id, steps, warmup, scale=None):
     reads, paired = numpy_sample(cfg_id, sc)
     n_raw = len(reads)
     sample = f"{NAMES[cfg_id]} at scale {sc} ({n_raw} raw reads, same coverage; generated with numpy, same read model)"
-    if not have_reference() and os.path.isdir("/root/reference/MetaGenomics"):
-        subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "ref"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
     times, n_unique, e_final = [], 0, 0
     host_cores = os.cpu_count() or 1
     if have_reference():
@@ -271,6 +277,45 @@ def golden_for(cfg_id, scale):
     return None
 
 
+DUMP_SEED = 20250601
+DUMP_EDGE_ROWS = 1 << 20      # 32 MiB of float64 edge rows
+DUMP_READS = 1 << 21          # 16 MiB of float64 superReadIDs
+
+
+def seeded_positions(n, cap):
+    """All of 0..n-1, or `cap` of them drawn with a fixed seed (the same positions for the same n), ascending."""
+    if n <= cap:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=cap, replace=False))
+
+
+def u64_limbs(words):
+    """64-bit words -> float64 16-bit limbs (low first): exact in float64."""
+    return np.array([(int(w) >> s) & 0xFFFF for w in words for s in (0, 16, 32, 48)], dtype=np.float64)
+
+
+def dump_outputs(out_dir, L, ctx, n_unique, st):
+    """What the last timed step left on the device, downloaded as a caller of the C ABI receives it (see the module docstring)."""
+    from metagenomics_b200._lib import check
+    from metagenomics_b200.api import EDGE_DTYPE
+    os.makedirs(out_dir, exist_ok=True)
+    n = C.c_uint64()
+    check(L.ogb_graph_edge_count(ctx._h, 0, C.byref(n)))
+    edges = np.zeros(n.value, dtype=EDGE_DTYPE)
+    check(L.ogb_graph_edges(ctx._h, 0, edges.ctypes.data, n.value))
+    rows = edges[seeded_positions(len(edges), DUMP_EDGE_ROWS)]
+    np.save(os.path.join(out_dir, "edges.npy"), np.stack([rows[k].astype(np.float64) for k in ("src", "dst", "offset", "orient")], axis=1))
+    del edges, rows
+    sup = np.zeros(n_unique + 1, dtype=np.uint64)
+    check(L.ogb_super_read_ids(ctx._h, sup.ctypes.data, n_unique + 1))
+    np.save(os.path.join(out_dir, "super_read_ids.npy"), sup[1:][seeded_positions(n_unique, DUMP_READS)].astype(np.float64))
+    gx, gs = C.c_uint64(), C.c_uint64()
+    check(L.ogb_graph_checksum(ctx._h, 0, C.byref(gx), C.byref(gs)))
+    np.save(os.path.join(out_dir, "edge_checksum.npy"), u64_limbs([gx.value, gs.value]))
+    np.save(os.path.join(out_dir, "counts.npy"),
+            np.array([n_unique, st["edges_pre"], n.value, st["nodes_final"], st["n_contained"]], dtype=np.float64))
+
+
 def next_pow2(x):
     p = 1 << 20
     while p < x:
@@ -287,7 +332,12 @@ def main():
     ap.add_argument("--config", type=int, default=3)
     ap.add_argument("--scale", type=float, default=1.0, help="scale of the configuration per GPU (weak scaling multiplies it by the GPU count)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (see above)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -298,9 +348,6 @@ def main():
         return
 
     args.warmup = max(args.warmup, 3)         # timing rule: at least three warm-up steps
-    import __graft_entry__ as g
-    if rank == 0:
-        g.build(quiet=True)
 
     import torch
     import torch.distributed as dist
@@ -309,7 +356,6 @@ def main():
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-        dist.barrier()                        # rank 0 has built the library
     from metagenomics_b200 import Context, Dataset, nccl_unique_id
     from metagenomics_b200._lib import check, lib
     from metagenomics_b200.api import EDGE_DTYPE
@@ -449,6 +495,8 @@ def main():
     st = ctx.stats()
     ms_step = float(per_step.mean())
     value = n_unique / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, L, ctx, n_unique, st)
 
     # ---- parity of the timed configuration: counters + checksum of the final edge set against the oracle's golden
     gx, gs = C.c_uint64(), C.c_uint64()
