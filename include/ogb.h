@@ -302,6 +302,52 @@ int ogb_graph_simplify(ogb_context *ctx, ogb_simplify_stats *stats);
  * by list_start. Capacities in elements (ogb_simplify_stats.n_edges_out / n_items). */
 int ogb_graph_composite_edges(ogb_context *ctx, ogb_cedge *edges, uint64_t edge_cap, ogb_clist_item *items, uint64_t item_cap);
 
+/* ----------------------------------------------------------------------------------------------
+ * Unitig sequences: OverlapGraph::getStringInEdge (OverlapGraph.cpp:2009) for the composite edges of the simplified graph, on the
+ * device (csrc/ogb_spell.cuh). Edge e = (src, dst, orient, offset) with items k = 1..c stands for reads src, item reads, dst;
+ * src is taken forward iff orient is 2 or 3, dst iff orient is 1 or 3, item k iff its orient is 1; they sit at P_0 = 0,
+ * P_k = sum of the first k item offsets, P_{c+1} = offset. The sequence has offset + length(dst) bases, base p taken from the
+ * read with the largest P_k <= p. Canonical unitigs are the edges saveGraphToFile writes (OverlapGraph.cpp:321-326): src < dst,
+ * or src == dst and index < twin.
+ * -------------------------------------------------------------------------------------------- */
+
+/* One spelled unitig. The sequences are laid out word-aligned: unitig i occupies packed words [start/32, start/32 + ceil(length/32))
+ * (2-bit, base p in bits 63-2(p%32) .. 62-2(p%32) of word p/32, A0 C1 G2 T3, unused bits zero), or bytes [start, start + length)
+ * of the ASCII form (32 bytes per word; the bytes after a unitig's end up to its next word are padding). */
+typedef struct ogb_unitig {
+	uint32_t edge;        /* index into the ogb_graph_composite_edges order */
+	uint32_t src;
+	uint32_t dst;
+	uint8_t orient;
+	uint8_t reserved[3];
+	uint64_t length;      /* bases */
+	uint64_t start;       /* in bases of the word-aligned layout: a multiple of 32 */
+} ogb_unitig; /* 32 bytes */
+
+typedef struct ogb_spell_stats {
+	uint64_t unitigs;     /* spelled by the last ogb_graph_spell */
+	uint64_t bases;
+	uint64_t words;       /* packed output words (ASCII: 32 bytes each) */
+	uint32_t launches;
+	float ms;             /* device time of ogb_graph_spell */
+} ogb_spell_stats;
+
+/* OverlapGraph::getStringInEdge (OverlapGraph.cpp:2009) for unitigs [first, first + count) of the selected edges (all, or the
+ * canonical ones with canonical_only != 0) in edge order; count = UINT64_MAX: all from first on. Several ranks can split the
+ * unitigs by range with no collective: every rank holds the whole simplified graph. The result stays on the device until the next
+ * upload, build, simplify or spell. Needs ogb_graph_simplify on the reads still uploaded (OGB_E_STATE otherwise); first beyond the
+ * number of selected edges is OGB_E_ARG. */
+int ogb_graph_spell(ogb_context *ctx, int canonical_only, uint64_t first, uint64_t count, ogb_spell_stats *stats);
+/* Copies the records of the last ogb_graph_spell and the sequences: packed words (out_cap in bytes >= 8 * words) or, ascii != 0,
+ * ACGT bytes decoded on the device (out_cap >= 32 * words). OGB_E_CAPACITY names the sizes needed (ogb_spell_stats.unitigs /
+ * words) when a buffer is too small. */
+int ogb_graph_unitigs(ogb_context *ctx, ogb_unitig *recs, uint64_t rec_cap, void *out, uint64_t out_cap, int ascii);
+/* Writes the unitigs of the last ogb_graph_spell as FASTA, one record per unitig in record order, the sequence on one line:
+ *     >unitig_<i> src=<src> dst=<dst> orient=<o> reads=<c+2> length=<L>
+ * (i = first + position in the range, c = reads inside the edge). Decoded on the device in bounded chunks staged through pinned
+ * host memory. No unitigs: an empty file. OGB_E_IO when the file cannot be written. */
+int ogb_graph_write_unitigs(ogb_context *ctx, const char *path);
+
 int ogb_get_stats(ogb_context *ctx, ogb_stats *out);
 
 /* Measurement helpers: CUDA events on the context's stream (the stream every kernel of this library

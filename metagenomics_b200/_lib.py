@@ -49,6 +49,14 @@ class SimplifyStats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_ if n != "reserved"}
 
 
+class SpellStats(C.Structure):
+    """ogb_spell_stats (include/ogb.h)."""
+    _fields_ = [(n, C.c_uint64) for n in ("unitigs", "bases", "words")] + [("launches", C.c_uint32), ("ms", C.c_float)]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
 # every symbol include/ogb.h declares: name -> (restype, argtypes)
 _u64p = C.POINTER(C.c_uint64)
 _vp = C.c_void_p
@@ -95,6 +103,9 @@ PROTOTYPES = {
     "ogb_graph_checksum": (C.c_int, [_vp, C.c_int, _u64p, _u64p]),
     "ogb_graph_simplify": (C.c_int, [_vp, C.POINTER(SimplifyStats)]),
     "ogb_graph_composite_edges": (C.c_int, [_vp, _vp, C.c_uint64, _vp, C.c_uint64]),
+    "ogb_graph_spell": (C.c_int, [_vp, C.c_int, C.c_uint64, C.c_uint64, C.POINTER(SpellStats)]),
+    "ogb_graph_unitigs": (C.c_int, [_vp, _vp, C.c_uint64, _vp, C.c_uint64, C.c_int]),
+    "ogb_graph_write_unitigs": (C.c_int, [_vp, C.c_char_p]),
     "ogb_get_stats": (C.c_int, [_vp, C.POINTER(Stats)]),
     "ogb_timer_begin": (C.c_int, [_vp]),
     "ogb_timer_end": (C.c_int, [_vp, C.POINTER(C.c_float)]),

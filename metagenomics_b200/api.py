@@ -17,7 +17,9 @@ EDGE_DTYPE = np.dtype([("src", "<u4"), ("dst", "<u4"), ("offset", "<u2"), ("orie
 CEDGE_DTYPE = np.dtype([("src", "<u4"), ("dst", "<u4"), ("offset", "<u8"), ("list_start", "<u8"), ("count", "<u4"), ("twin", "<u4"), ("orient", "u1"),
                         ("reserved", "u1", (3,)), ("reserved2", "<u4")])
 CITEM_DTYPE = np.dtype([("read", "<u4"), ("offset", "<u2"), ("orient", "u1"), ("reserved", "u1")])
-assert CEDGE_DTYPE.itemsize == 40 and CITEM_DTYPE.itemsize == 8
+# ogb_unitig: one spelled unitig; its sequence is bases [start, start + length) of the word-aligned layout (OverlapGraph.unitigs)
+UNITIG_DTYPE = np.dtype([("edge", "<u4"), ("src", "<u4"), ("dst", "<u4"), ("orient", "u1"), ("reserved", "u1", (3,)), ("length", "<u8"), ("start", "<u8")])
+assert CEDGE_DTYPE.itemsize == 40 and CITEM_DTYPE.itemsize == 8 and UNITIG_DTYPE.itemsize == 32
 assert EDGE_DTYPE.itemsize == C.sizeof(Edge) == 12
 
 
@@ -247,6 +249,31 @@ class OverlapGraph:
         items = np.zeros(st.n_items, dtype=CITEM_DTYPE)
         check(lib().ogb_graph_composite_edges(self.ctx._h, edges.ctypes.data, len(edges), items.ctypes.data, len(items)))
         return edges, items, st.as_dict()
+
+    def spell(self, canonical=True, first=0, count=None):
+        """Spells unitigs [first, first + count) of the simplified graph's edges (the canonical ones, src < dst or a self-edge's first
+        half, with canonical=True; count None = all) on the device -- the sequences getStringInEdge (OverlapGraph.cpp:2009) returns.
+        Needs simplify() first. The result stays on the device; returns the ogb_spell_stats as a dict."""
+        from ._lib import SpellStats
+        st = SpellStats()
+        check(lib().ogb_graph_spell(self.ctx._h, 1 if canonical else 0, int(first), 2**64 - 1 if count is None else int(count), C.byref(st)))
+        return st.as_dict()
+
+    def unitigs(self, canonical=True, ascii=True, first=0, count=None):
+        """(records, sequences): records as UNITIG_DTYPE in edge order; sequences one flat buffer in which unitig i is
+        sequences[start : start + length] -- uint8 ACGT bytes with ascii=True, else the packed uint64 words (2-bit, base p of a
+        unitig in bits 63-2(p%32) .. 62-2(p%32) of word start/32 + p/32)."""
+        st = self.spell(canonical, first, count)
+        recs = np.zeros(st["unitigs"], dtype=UNITIG_DTYPE)
+        out = np.zeros(st["words"] * 32, dtype=np.uint8) if ascii else np.zeros(st["words"], dtype=np.uint64)
+        check(lib().ogb_graph_unitigs(self.ctx._h, recs.ctypes.data, len(recs), out.ctypes.data, out.nbytes, 1 if ascii else 0))
+        return recs, out
+
+    def write_unitigs(self, path, canonical=True):
+        """Spells the (canonical) unitigs and writes them as FASTA (ogb_graph_write_unitigs); returns the spell stats."""
+        st = self.spell(canonical)
+        check(lib().ogb_graph_write_unitigs(self.ctx._h, str(path).encode()))
+        return st
 
     def checksum(self, pre=False):
         """[xor, sum] of the 64-bit mix of every edge tuple, computed on the device (the figure of tests/golden/full_size.json)."""

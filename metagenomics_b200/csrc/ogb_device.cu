@@ -11,6 +11,7 @@
 #include "ogb_internal.h"
 #include "ogb_kernels.cuh"
 #include "ogb_contract.cuh"
+#include "ogb_spell.cuh"
 
 #include <algorithm>
 #include <chrono>
@@ -191,7 +192,16 @@ struct ogb_context {
 	Pool<ogb_cedge> s_out;
 	Pool<ogb_clist_item> s_out_items;
 	bool have_simplified = false;
+	uint64_t s_stamp = 0;            // reads_stamp of the reads the simplified graph was built on
 	ogb_simplify_stats sst = {};
+	// unitig sequences (ogb_spell.cuh): selection and item scans, records, packed words, ASCII scratch
+	Pool<u32> sp_sel, sp_ioff, sp_nw;
+	Pool<u64> sp_rank, sp_ipos, sp_wpos, sp_words;
+	Pool<ogb_unitig> sp_rec;
+	Pool<char> sp_ascii;
+	bool have_spelled = false;
+	u64 sp_first = 0;
+	ogb_spell_stats spst = {};
 	// L2 persistence window on the bucket summary (l2_keep_summary)
 	const void *l2_window_ptr = nullptr;
 	size_t l2_window_bytes = 0;
@@ -366,6 +376,8 @@ extern "C" void ogb_context_destroy(ogb_context *c)
 	c->scratch_keys.release(); c->fin.release(); c->pre.release(); c->flush.release(); c->fin_stage.release();
 	c->sE.release(); c->s_rec.release(); c->s_rowptr.release(); c->s_cp.release(); c->s_info.release(); c->s_list.release(); c->s_keep.release(); c->s_items.release(); c->s_blocker.release();
 	c->s_state.release(); c->s_ready.release(); c->s_flag.release(); c->s_epos.release(); c->s_lpos.release(); c->s_ctr.release(); c->s_out.release(); c->s_out_items.release();
+	c->sp_sel.release(); c->sp_ioff.release(); c->sp_nw.release(); c->sp_rank.release(); c->sp_ipos.release(); c->sp_wpos.release(); c->sp_words.release();
+	c->sp_rec.release(); c->sp_ascii.release();
 	if (c->d_ctr) cudaFree(c->d_ctr);
 	if (c->d_tot) cudaFree(c->d_tot);
 	if (c->d_cursor) cudaFree(c->d_cursor);
@@ -445,7 +457,7 @@ static int upload_common(ogb_context *c, u64 total_words, const std::vector<u64>
 	}
 	c->slot_cap = 64;
 	c->reads_stamp++;
-	c->have_reads = true; c->have_table = false; c->contain_done = false; c->any_contained = false; c->have_graph = false; c->have_pre = false;
+	c->have_reads = true; c->have_table = false; c->contain_done = false; c->any_contained = false; c->have_graph = false; c->have_pre = false; c->have_spelled = false;
 	return OGB_OK;
 }
 
@@ -1398,7 +1410,7 @@ extern "C" int ogb_build_graph(ogb_context *c, int keep_pre)
 	OGB_TRY(l2_keep_summary(c, true));                                      // (a second build on the same index: the first one closed the window)
 	// buildOverlapGraphFromHashTable always marks contained reads first (OverlapGraph.cpp:140)
 	if (!c->contain_done) OGB_TRY(ogb_mark_contained(c));
-	c->have_graph = false; c->have_pre = false; c->have_simplified = false; c->n_final = 0; c->n_pre = 0;
+	c->have_graph = false; c->have_pre = false; c->have_simplified = false; c->have_spelled = false; c->n_final = 0; c->n_pre = 0;
 	const u32 n = c->n;
 	if (n == 0) { c->have_graph = true; c->have_pre = keep_pre != 0; c->st.edges_pre = c->st.edges_pre_local = c->st.edges_final = c->st.nodes_final = 0; return OGB_OK; }
 	u32 lo, hi;
@@ -1739,7 +1751,7 @@ extern "C" int ogb_graph_simplify(ogb_context *c, ogb_simplify_stats *stats)
 	const u64 ne = c->n_final;
 	const u32 n = c->n;
 	if (ne >= (1ull << 31) || n >= (1u << 30)) { ogb_set_error("ogb_graph_simplify: %llu edges / %u reads exceed the 31-bit entry and record indices", (unsigned long long)ne, n); return OGB_E_CAPACITY; }
-	c->have_simplified = false;
+	c->have_simplified = false; c->have_spelled = false;
 	ogb_simplify_stats st = {};
 	st.n_edges_in = ne;
 	const u64 nrec = 2 * ((u64)n + 1);
@@ -1853,7 +1865,7 @@ extern "C" int ogb_graph_simplify(ogb_context *c, ogb_simplify_stats *stats)
 	}
 	st.ms_lists = st.ms - st.ms_setup - st.ms_sweeps - st.ms_dead_ends;
 	st.n_edges_out = n_out; st.n_items = n_items;
-	c->sst = st; c->have_simplified = true;
+	c->sst = st; c->have_simplified = true; c->s_stamp = c->reads_stamp;
 	if (stats) *stats = st;
 	return OGB_OK;
 }
@@ -1872,6 +1884,157 @@ extern "C" int ogb_graph_composite_edges(ogb_context *c, ogb_cedge *edges, uint6
 	if (ni) CUDA_TRY(cudaMemcpyAsync(items, c->s_out_items.p, ni * sizeof(ogb_clist_item), cudaMemcpyDeviceToHost, c->stream));
 	CUDA_TRY(cudaStreamSynchronize(c->stream));
 	return OGB_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Unitig sequences (OverlapGraph::getStringInEdge, OverlapGraph.cpp:2009): see ogb_spell.cuh.
+// ------------------------------------------------------------------------------------------------
+static SpellArgs spell_args(const ogb_context *c)
+{
+	SpellArgs A;
+	A.words = c->words.p; A.meta = c->uniform_len ? nullptr : c->meta.p; A.uniform_len = c->uniform_len; A.uniform_pw = c->uniform_pw;
+	A.edges = c->s_out.p; A.items = c->s_out_items.p; A.ipos = c->sp_ipos.p; A.rec = c->sp_rec.p; A.n_rec = c->spst.unitigs; A.wpos = c->sp_wpos.p;
+	return A;
+}
+
+extern "C" int ogb_graph_spell(ogb_context *c, int canonical_only, uint64_t first, uint64_t count, ogb_spell_stats *stats)
+{
+	if (!c) { ogb_set_error("ogb_graph_spell: NULL context"); return OGB_E_ARG; }
+	if (!c->have_simplified || c->s_stamp != c->reads_stamp) { ogb_set_error("ogb_graph_spell: run ogb_graph_simplify on the uploaded reads first"); return OGB_E_STATE; }
+	CUDA_TRY(cudaSetDevice(c->device));
+	c->have_spelled = false;
+	const u64 ne = c->sst.n_edges_out, ni = c->sst.n_items, cap = std::min<u64>(count, ne);
+	ogb_spell_stats st = {};
+	const int grid_max = c->sm_count * 8;
+	auto grid = [&](u64 items) { return (unsigned)std::max<u64>(1, std::min<u64>((items + 255) / 256, (u64)grid_max)); };
+	OGB_TRY(c->sp_sel.ensure(std::max<u64>(ne, 1))); OGB_TRY(c->sp_rank.ensure(ne + 1));
+	OGB_TRY(c->sp_ioff.ensure(std::max<u64>(ni, 1))); OGB_TRY(c->sp_ipos.ensure(ni + 1));
+	OGB_TRY(c->sp_rec.ensure(std::max<u64>(cap, 1))); OGB_TRY(c->sp_nw.ensure(std::max<u64>(cap, 1))); OGB_TRY(c->sp_wpos.ensure(cap + 1));
+	OGB_TRY(c->s_ctr.ensure(16));
+	u64 *ctr = c->s_ctr.p;
+	CUDA_TRY(cudaEventRecord(c->ev[EV_T0], c->stream));
+	CUDA_TRY(cudaMemsetAsync(ctr, 0, 2 * sizeof(u64), c->stream));                // [0] selected edges, [1] bases
+	CUDA_TRY(cudaMemsetAsync(c->sp_ipos.p + ni, 0, sizeof(u64), c->stream));
+	CUDA_TRY(cudaMemsetAsync(c->sp_wpos.p + cap, 0, sizeof(u64), c->stream));
+	SpellArgs A = spell_args(c);
+	if (ne) {
+		k_sp_select<<<grid(ne), 256, 0, c->stream>>>(c->s_out.p, ne, canonical_only, c->sp_sel.p);
+		st.launches++;
+		OGB_TRY(exclusive_scan(c, c->sp_sel.p, (u32)ne, c->sp_rank.p, ctr, nullptr, nullptr));
+		st.launches += 3;
+	}
+	if (ni) {
+		k_sp_item_offsets<<<grid(ni), 256, 0, c->stream>>>(c->s_out_items.p, ni, c->sp_ioff.p);
+		st.launches++;
+		OGB_TRY(exclusive_scan(c, c->sp_ioff.p, (u32)ni, c->sp_ipos.p, c->sp_ipos.p + ni, nullptr, nullptr));
+		st.launches += 3;
+	}
+	if (cap) {
+		CUDA_TRY(cudaMemsetAsync(c->sp_nw.p, 0, cap * sizeof(u32), c->stream));       // the range may end before cap records
+		k_sp_records<<<grid(ne), 256, 0, c->stream>>>(A, ne, c->sp_sel.p, c->sp_rank.p, first, cap, c->sp_rec.p, c->sp_nw.p, ctr + 1);
+		st.launches++;
+		OGB_TRY(exclusive_scan(c, c->sp_nw.p, (u32)cap, c->sp_wpos.p, c->sp_wpos.p + cap, nullptr, nullptr));
+		st.launches += 3;
+	}
+	CUDA_TRY(cudaGetLastError());
+	u64 h[3] = {0, 0, 0};
+	CUDA_TRY(cudaMemcpyAsync(h, ctr, 2 * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(h + 2, c->sp_wpos.p + cap, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaStreamSynchronize(c->stream));
+	const u64 n_sel = h[0];
+	if (first > n_sel) { ogb_set_error("ogb_graph_spell: first unitig %llu beyond the %llu selected", (unsigned long long)first, (unsigned long long)n_sel); return OGB_E_ARG; }
+	st.unitigs = std::min<u64>(cap, n_sel - first);
+	st.bases = h[1]; st.words = h[2];
+	c->spst = st;
+	OGB_TRY(c->sp_words.ensure(std::max<u64>(st.words, 1)));
+	if (st.words) {
+		A = spell_args(c);
+		k_spell_words<<<grid(st.words), 256, 0, c->stream>>>(A, st.words, c->sp_rec.p, c->sp_words.p);
+		CUDA_TRY(cudaGetLastError());
+		st.launches++;
+	}
+	CUDA_TRY(cudaEventRecord(c->ev[EV_T1], c->stream));
+	CUDA_TRY(cudaStreamSynchronize(c->stream));
+	CUDA_TRY(cudaEventElapsedTime(&st.ms, c->ev[EV_T0], c->ev[EV_T1]));
+	c->spst = st;
+	c->sp_first = first;
+	c->have_spelled = true;
+	if (stats) *stats = c->spst;
+	return OGB_OK;
+}
+
+extern "C" int ogb_graph_unitigs(ogb_context *c, ogb_unitig *recs, uint64_t rec_cap, void *out, uint64_t out_cap, int ascii)
+{
+	if (!c) { ogb_set_error("ogb_graph_unitigs: NULL context"); return OGB_E_ARG; }
+	if (!c->have_spelled) { ogb_set_error("ogb_graph_unitigs: run ogb_graph_spell first"); return OGB_E_STATE; }
+	const u64 nu = c->spst.unitigs, nw = c->spst.words, bytes = nw * (ascii ? 32 : 8);
+	if ((nu && (!recs || rec_cap < nu)) || (bytes && (!out || out_cap < bytes))) {
+		ogb_set_error("ogb_graph_unitigs: need room for %llu records and %llu bytes (%llu words%s)", (unsigned long long)nu, (unsigned long long)bytes,
+		              (unsigned long long)nw, ascii ? " x 32 ASCII bytes" : "");
+		return OGB_E_CAPACITY;
+	}
+	CUDA_TRY(cudaSetDevice(c->device));
+	if (nu) CUDA_TRY(cudaMemcpyAsync(recs, c->sp_rec.p, nu * sizeof(ogb_unitig), cudaMemcpyDeviceToHost, c->stream));
+	if (nw && !ascii) CUDA_TRY(cudaMemcpyAsync(out, c->sp_words.p, bytes, cudaMemcpyDeviceToHost, c->stream));
+	if (nw && ascii) {
+		OGB_TRY(c->sp_ascii.ensure(bytes));
+		k_spell_ascii<<<(unsigned)std::min<u64>((nw + 255) / 256, (u64)c->sm_count * 8), 256, 0, c->stream>>>(c->sp_words.p, 0, nw, c->sp_ascii.p);
+		CUDA_TRY(cudaGetLastError());
+		CUDA_TRY(cudaMemcpyAsync(out, c->sp_ascii.p, bytes, cudaMemcpyDeviceToHost, c->stream));
+	}
+	CUDA_TRY(cudaStreamSynchronize(c->stream));
+	return OGB_OK;
+}
+
+// The FASTA writer: chunks of OGB_SPELL_CHUNK words are decoded on the device and staged through pinned memory; a record's header is
+// written when its first base arrives, so a unitig longer than a chunk spans several.
+enum { OGB_SPELL_CHUNK = 1 << 20 };   // 32 MB of ASCII per chunk
+extern "C" int ogb_graph_write_unitigs(ogb_context *c, const char *path)
+{
+	if (!c || !path) { ogb_set_error("ogb_graph_write_unitigs: NULL argument"); return OGB_E_ARG; }
+	if (!c->have_spelled) { ogb_set_error("ogb_graph_write_unitigs: run ogb_graph_spell first"); return OGB_E_STATE; }
+	CUDA_TRY(cudaSetDevice(c->device));
+	const u64 nu = c->spst.unitigs, nw = c->spst.words, ne = c->sst.n_edges_out;
+	std::vector<ogb_unitig> rec(nu);
+	std::vector<ogb_cedge> edges(nu ? ne : 0);                                 // for the read counts of the headers
+	if (nu) {
+		CUDA_TRY(cudaMemcpyAsync(rec.data(), c->sp_rec.p, nu * sizeof(ogb_unitig), cudaMemcpyDeviceToHost, c->stream));
+		CUDA_TRY(cudaMemcpyAsync(edges.data(), c->s_out.p, ne * sizeof(ogb_cedge), cudaMemcpyDeviceToHost, c->stream));
+		CUDA_TRY(cudaStreamSynchronize(c->stream));
+	}
+	FILE *f = fopen(path, "wb");
+	if (!f) { ogb_set_error("ogb_graph_write_unitigs: cannot open %s for writing", path); return OGB_E_IO; }
+	char *stage = nullptr;
+	int rc = OGB_OK;
+	auto body = [&]() -> int {
+		if (!nw) return OGB_OK;
+		const u64 chunk = std::min<u64>(nw, OGB_SPELL_CHUNK);
+		OGB_TRY(c->sp_ascii.ensure(chunk * 32));
+		CUDA_TRY(cudaMallocHost((void **)&stage, chunk * 32));
+		u64 r = 0;                                                               // record whose bases come next
+		for (u64 w0 = 0; w0 < nw; w0 += chunk) {
+			const u64 w1 = std::min(nw, w0 + chunk);
+			k_spell_ascii<<<(unsigned)std::min<u64>((w1 - w0 + 255) / 256, (u64)c->sm_count * 8), 256, 0, c->stream>>>(c->sp_words.p, w0, w1, c->sp_ascii.p);
+			CUDA_TRY(cudaGetLastError());
+			CUDA_TRY(cudaMemcpyAsync(stage, c->sp_ascii.p, (w1 - w0) * 32, cudaMemcpyDeviceToHost, c->stream));
+			CUDA_TRY(cudaStreamSynchronize(c->stream));
+			const u64 b0 = 32 * w0, b1 = 32 * w1;                                // bases of the word-aligned layout in the stage
+			for (; r < nu && rec[r].start < b1; r++) {
+				const ogb_unitig &u = rec[r];
+				const u64 a = std::max<u64>(u.start, b0), b = std::min<u64>(u.start + u.length, b1);
+				if (a == u.start) fprintf(f, ">unitig_%llu src=%u dst=%u orient=%u reads=%u length=%llu\n", (unsigned long long)(c->sp_first + r), u.src, u.dst,
+				                           (unsigned)u.orient, edges[u.edge].count + 2, (unsigned long long)u.length);
+				if (b > a && fwrite(stage + (a - b0), 1, b - a, f) != b - a) { ogb_set_error("ogb_graph_write_unitigs: write to %s failed", path); return OGB_E_IO; }
+				if (u.start + u.length > b1) break;                              // continues in the next chunk
+				fputc('\n', f);
+			}
+		}
+		return OGB_OK;
+	};
+	rc = body();
+	if (stage) cudaFreeHost(stage);
+	if (fclose(f) != 0 && rc == OGB_OK) { ogb_set_error("ogb_graph_write_unitigs: closing %s failed", path); rc = OGB_E_IO; }
+	return rc;
 }
 
 extern "C" int ogb_get_stats(ogb_context *c, ogb_stats *out)

@@ -20,6 +20,19 @@ def shard_bounds(n, rank, world):
     return min(n, per * rank), min(n, per * (rank + 1))
 
 
+def unitig_range(edges, rank, world, canonical=True):
+    """(first, count) of the unitigs `rank` spells (OverlapGraph.spell / unitigs) given the simplified graph's edges
+    (OverlapGraph.simplify()): the contiguous ranges of shard_bounds over the selected edges. Every rank holds the whole simplified
+    graph, so the split needs no collective."""
+    import numpy as np
+    n = len(edges)
+    if canonical:
+        i = np.arange(n)
+        n = int(((edges["src"] < edges["dst"]) | ((edges["src"] == edges["dst"]) & (i < edges["twin"]))).sum())
+    lo, hi = shard_bounds(n, rank, world)
+    return lo, hi - lo
+
+
 def broadcast_bytes(payload, src=0):
     """Broadcasts a bytes object made on `src` (the 128-byte ncclUniqueId) to every rank."""
     box = [payload if dist.get_rank() == src else None]

@@ -8,12 +8,14 @@ static bool byDestination(Edge *a, Edge *b) { return a->getDestinationRead()->ge
 static bool byOffset(Edge *a, Edge *b) { return a->getOverlapOffset() < b->getOverlapOffset(); }
 
 bool OverlapGraph::simplifyInBuild = true;
+bool OverlapGraph::spellInBuild = false;
 
 OverlapGraph::OverlapGraph(void)
 	: dataSet(NULL), hashTable(NULL), graph(new vector<vector<Edge *> *>), numberOfNodes(0), numberOfEdges(0), hashStringLength(0), flowComputed(false)
 {
 	memset(&lastStats, 0, sizeof lastStats);
 	memset(&lastSimplifyStats, 0, sizeof lastSimplifyStats);
+	memset(&lastSpellStats, 0, sizeof lastSpellStats);
 }
 
 OverlapGraph::OverlapGraph(HashTable *ht)
@@ -21,6 +23,7 @@ OverlapGraph::OverlapGraph(HashTable *ht)
 {
 	memset(&lastStats, 0, sizeof lastStats);
 	memset(&lastSimplifyStats, 0, sizeof lastSimplifyStats);
+	memset(&lastSpellStats, 0, sizeof lastSpellStats);
 	buildOverlapGraphFromHashTable(ht);
 }
 
@@ -109,7 +112,21 @@ bool OverlapGraph::simplifyGraph(void)
 		insertEdge(objs[e]);
 	}
 	for (uint64_t e = 0; e < ne; e++) objs[e]->setReverseEdge(objs[edges[e].twin]);
+	if (spellInBuild) {														// the sequences of the canonical unitigs (getStringInEdge, :2009)
+		ogbCheck(ogb_graph_spell(ctx, 1, 0, UINT64_MAX, &lastSpellStats), "OverlapGraph::simplifyGraph");
+		return true;														// they stay on the device, with the table, until saveUnitigsToFile
+	}
 	delete hashTable;														// :210 -- the graph owns and frees the table
+	hashTable = NULL;
+	return true;
+}
+
+// The unitigs simplifyGraph() spelled (spellInBuild) as FASTA, decoded on the device; then the table and its context go, as at :210.
+bool OverlapGraph::saveUnitigsToFile(string fileName)
+{
+	if (!hashTable) throw OgbFailure(OGB_E_STATE, "saveUnitigsToFile: no unitigs on the device (set OverlapGraph::spellInBuild before the build)");
+	ogbCheck(ogb_graph_write_unitigs(hashTable->getContext(), fileName.c_str()), "OverlapGraph::saveUnitigsToFile");
+	delete hashTable;
 	hashTable = NULL;
 	return true;
 }

@@ -40,10 +40,13 @@ class OverlapGraph
 		void materialise(const ogb_edge *edges, UINT64 n);
 		void clearGraph(void);
 		ogb_simplify_stats lastSimplifyStats;
+		ogb_spell_stats lastSpellStats;
 
 	public:
 		bool flowComputed;
 		static bool simplifyInBuild;					// true (default): the build ends with the fix-point of :211-215, like the reference's
+		static bool spellInBuild;						// false (default); true: simplifyGraph() also spells the canonical unitigs on the device
+														// (getStringInEdge, :2009) and keeps the hash table's device context for saveUnitigsToFile
 		OverlapGraph(void);
 		OverlapGraph(HashTable *ht);
 		~OverlapGraph();
@@ -62,12 +65,14 @@ class OverlapGraph
 		bool setDataset(Dataset *dataset) { dataSet = dataset; dataset->readMatePairsFromFile(); return true; }
 		void sortEdges();
 		bool saveGraphToFile(string fileName);			// OverlapGraph.cpp:1219-1259: the reference's .unitig text format
+		bool saveUnitigsToFile(string fileName);		// the unitigs spelled in the build as FASTA (ogb_graph_write_unitigs); frees the hash table
 		bool readGraphFromFile(string fileName);		// OverlapGraph.cpp:1267-1367 (resume path, main.cpp:36-42)
 		Edge *findEdge(UINT64 source, UINT64 destination);
 		bool isEdgePresent(UINT64 source, UINT64 destination);
 		vector<vector<Edge *> *> *getGraph(void) { return graph; }
 		const ogb_stats &getBuildStats(void) const { return lastStats; }
 		const ogb_simplify_stats &getSimplifyStats(void) const { return lastSimplifyStats; }
+		const ogb_spell_stats &getSpellStats(void) const { return lastSpellStats; }
 };
 
 #endif

@@ -4,10 +4,11 @@
 // (calculateFlow, the three simplification loops, printGraph) is host code that consumes the graph
 // this program produces and is not part of this library.
 //
-//   ogb_overlap -l minOverlap [-se n files...] [-pe n files...] [-f prefix] [--dump file]
+//   ogb_overlap -l minOverlap [-se n files...] [-pe n files...] [-f prefix] [--dump file] [--unitigs file]
 //
 // --dump writes the graph in the binary format the parity tests read, so one comparator reads
-// the output of the unmodified reference and of this program.
+// the output of the unmodified reference and of this program. --unitigs writes the sequences of the canonical unitigs of the
+// simplified graph as FASTA, spelled on the device (OverlapGraph::spellInBuild, saveUnitigsToFile).
 #include "Common.h"
 #include "Dataset.h"
 #include "Edge.h"
@@ -80,7 +81,7 @@ int main(int argc, char **argv)
 	UINT64 minimumOverlapLength = 0;
 	vector<string> pairedEndFileNames, singleEndFileNames;
 	string allFileName = "";
-	const char *dumpPath = NULL, *resavePath = NULL, *matesPath = NULL;
+	const char *dumpPath = NULL, *resavePath = NULL, *matesPath = NULL, *unitigsPath = NULL;
 	bool startFromUnitigGraph = false;
 	for (int i = 1; i < argc; i++) {
 		string a = argv[i];
@@ -93,13 +94,18 @@ int main(int argc, char **argv)
 		else if (a == "-s") startFromUnitigGraph = true;												// main.cpp: resume from <prefix>.unitig
 		else if (a == "--resave" && i + 1 < argc) resavePath = argv[++i];
 		else if (a == "--mates" && i + 1 < argc) matesPath = argv[++i];
+		else if (a == "--unitigs" && i + 1 < argc) unitigsPath = argv[++i];
 		else {
-			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file]" << endl;
+			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file] [--unitigs file]" << endl;
 			return a == "-h" || a == "--help" ? 0 : 1;
 		}
 	}
 	if (minimumOverlapLength == 0 || (pairedEndFileNames.empty() && singleEndFileNames.empty())) {
 		cerr << "ogb_overlap: need -l and at least one input file" << endl;
+		return 1;
+	}
+	if (startFromUnitigGraph && unitigsPath) {
+		cerr << "ogb_overlap: --unitigs needs the build on the device; -s resumes from a .unitig file without one" << endl;
 		return 1;
 	}
 	try {
@@ -119,6 +125,7 @@ int main(int argc, char **argv)
 			return 0;
 		}
 		if (dumpPath) OverlapGraph::simplifyInBuild = false;											// --dump wants the graph as it is at OverlapGraph.cpp:210
+		if (unitigsPath) OverlapGraph::spellInBuild = true;
 		HashTable *hashTable = new HashTable();															// main.cpp:45
 		hashTable->insertDataset(dataSet, minimumOverlapLength);										// main.cpp:46
 		overlapGraph = new OverlapGraph(hashTable); //hashTable deleted by this function after building the graph (main.cpp:47)
@@ -136,6 +143,11 @@ int main(int argc, char **argv)
 		     << " nodes: " << overlapGraph->getNumberOfNodes() << " edges: " << overlapGraph->getNumberOfEdges()
 		     << " device ms: " << st.ms_total << " + simplification " << ss.ms << " (" << ss.merges << " merges, " << ss.dead_ends << " dead ends, "
 		     << ss.iterations << " iterations, " << ss.rounds << " rounds)" << endl;
+		if (unitigsPath) {
+			overlapGraph->saveUnitigsToFile(unitigsPath);
+			const ogb_spell_stats &sp = overlapGraph->getSpellStats();
+			cout << "unitigs: " << sp.unitigs << " bases: " << sp.bases << " spell device ms: " << sp.ms << " (" << unitigsPath << ")" << endl;
+		}
 		delete dataSet;
 		delete overlapGraph;
 	} catch (const OgbFailure &e) {
