@@ -348,6 +348,58 @@ int ogb_graph_unitigs(ogb_context *ctx, ogb_unitig *recs, uint64_t rec_cap, void
  * host memory. No unitigs: an empty file. OGB_E_IO when the file cannot be written. */
 int ogb_graph_write_unitigs(ogb_context *ctx, const char *path);
 
+/* ----------------------------------------------------------------------------------------------
+ * Unitig coverage: per-base read depth of the unitigs of the last ogb_graph_spell, on the device (csrc/ogb_coverage.cuh).
+ * With f(r) the read's frequency (the Dataset's dedupe count), the depth D[p] of base p of a unitig is the sum of f(r_k) over
+ * its placements k (reads src, items, dst at P_k as above) with P_k <= p < P_k + length(r_k), plus f(x) for every contained read x
+ * whose superReadID is one of those reads, over the interval x occupies in it: q = the smallest shift at which x's stored strand
+ * occurs in the super read's forward strand, else the smallest at which its reverse complement does; the interval starts at
+ * P_k + q (super read forward in the unitig) or P_k + length(super) - q - length(x) (reverse). A twin's profile is the reverse.
+ * -------------------------------------------------------------------------------------------- */
+
+typedef struct ogb_unitig_coverage {
+	uint32_t edge;         /* as ogb_unitig.edge */
+	uint32_t reads;        /* placements: reads inside the edge + 2 */
+	uint32_t contained;    /* contained reads placed in the unitig */
+	uint32_t depth_min;
+	uint32_t depth_max;
+	uint32_t reserved;
+	uint64_t length;       /* as ogb_unitig.length / .start: the profile is depth[start .. start + length) */
+	uint64_t start;
+	uint64_t read_count;   /* sum of f over the placements and the contained reads placed */
+	uint64_t depth_sum;    /* sum of D over the bases (= sum of f * length over the same reads) */
+	uint64_t depth_sq_sum; /* sum of D^2, mod 2^64: exact while depth_max^2 * length < 2^64 */
+} ogb_unitig_coverage; /* 64 bytes */
+
+typedef struct ogb_coverage_stats {
+	uint64_t unitigs;
+	uint64_t bases;
+	uint64_t placements;            /* reads of the unitigs, src and dst included */
+	uint64_t contained_placements;  /* contained reads placed, over all unitigs */
+	uint64_t unplaced;              /* contained reads found in neither strand of their super read: 0 on a graph K2 verified */
+	uint32_t launches;
+	float ms;                       /* device time of ogb_graph_coverage */
+	float ms_locate;                /* upload of freq (from the caller's memory) and contained reads located in their super reads */
+	float ms_depth;                 /* placements into the difference array, and its scan */
+	float ms_reduce;                /* per-base profile and per-unitig sums */
+	uint32_t reserved;
+} ogb_coverage_stats; /* 64 bytes */
+
+/* The coverage of the unitigs of the last ogb_graph_spell (the same range and selection). freq = the frequency of every uploaded
+ * read by ID - 1 (n = the uploaded read count; anything else is OGB_E_ARG), copied to the device per call. No spell on the
+ * current reads: OGB_E_STATE. The result stays on the device until the next upload, build, simplify or spell. Integers only:
+ * two runs give the same bits. */
+int ogb_graph_coverage(ogb_context *ctx, const uint32_t *freq, uint64_t n, ogb_coverage_stats *stats);
+/* Copies the records of the last ogb_graph_coverage (rec_cap >= unitigs) and, when depth is not NULL, the u32 profile in the
+ * spell's word-aligned layout (depth_cap in elements >= 32 * ogb_spell_stats.words; padding bases are 0). OGB_E_CAPACITY names
+ * the sizes needed. */
+int ogb_graph_unitig_coverage(ogb_context *ctx, ogb_unitig_coverage *recs, uint64_t rec_cap, uint32_t *depth, uint64_t depth_cap);
+/* Writes the last ogb_graph_coverage as TSV: one '#' header line, then per unitig in record order
+ *     unitig_<i> src dst length reads contained read_count mean_depth sd_depth min_depth max_depth
+ * with i as in ogb_graph_write_unitigs (the names join with the FASTA), mean = depth_sum / length and
+ * sd = sqrt(max(0, depth_sq_sum / length - mean^2)) in double, printed %.4f. OGB_E_IO when the file cannot be written. */
+int ogb_graph_write_coverage(ogb_context *ctx, const char *path);
+
 int ogb_get_stats(ogb_context *ctx, ogb_stats *out);
 
 /* Measurement helpers: CUDA events on the context's stream (the stream every kernel of this library

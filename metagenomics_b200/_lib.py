@@ -57,6 +57,15 @@ class SpellStats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class CoverageStats(C.Structure):
+    """ogb_coverage_stats (include/ogb.h)."""
+    _fields_ = [(n, C.c_uint64) for n in ("unitigs", "bases", "placements", "contained_placements", "unplaced")] + [("launches", C.c_uint32)] + [
+        (n, C.c_float) for n in ("ms", "ms_locate", "ms_depth", "ms_reduce")] + [("reserved", C.c_uint32)]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_ if n != "reserved"}
+
+
 # every symbol include/ogb.h declares: name -> (restype, argtypes)
 _u64p = C.POINTER(C.c_uint64)
 _vp = C.c_void_p
@@ -106,6 +115,9 @@ PROTOTYPES = {
     "ogb_graph_spell": (C.c_int, [_vp, C.c_int, C.c_uint64, C.c_uint64, C.POINTER(SpellStats)]),
     "ogb_graph_unitigs": (C.c_int, [_vp, _vp, C.c_uint64, _vp, C.c_uint64, C.c_int]),
     "ogb_graph_write_unitigs": (C.c_int, [_vp, C.c_char_p]),
+    "ogb_graph_coverage": (C.c_int, [_vp, _vp, C.c_uint64, C.POINTER(CoverageStats)]),
+    "ogb_graph_unitig_coverage": (C.c_int, [_vp, _vp, C.c_uint64, _vp, C.c_uint64]),
+    "ogb_graph_write_coverage": (C.c_int, [_vp, C.c_char_p]),
     "ogb_get_stats": (C.c_int, [_vp, C.POINTER(Stats)]),
     "ogb_timer_begin": (C.c_int, [_vp]),
     "ogb_timer_end": (C.c_int, [_vp, C.POINTER(C.c_float)]),

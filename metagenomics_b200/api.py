@@ -19,7 +19,10 @@ CEDGE_DTYPE = np.dtype([("src", "<u4"), ("dst", "<u4"), ("offset", "<u8"), ("lis
 CITEM_DTYPE = np.dtype([("read", "<u4"), ("offset", "<u2"), ("orient", "u1"), ("reserved", "u1")])
 # ogb_unitig: one spelled unitig; its sequence is bases [start, start + length) of the word-aligned layout (OverlapGraph.unitigs)
 UNITIG_DTYPE = np.dtype([("edge", "<u4"), ("src", "<u4"), ("dst", "<u4"), ("orient", "u1"), ("reserved", "u1", (3,)), ("length", "<u8"), ("start", "<u8")])
-assert CEDGE_DTYPE.itemsize == 40 and CITEM_DTYPE.itemsize == 8 and UNITIG_DTYPE.itemsize == 32
+# ogb_unitig_coverage: the depth of a unitig is bases [start, start + length) of the flat profile (OverlapGraph.depth)
+COVERAGE_DTYPE = np.dtype([("edge", "<u4"), ("reads", "<u4"), ("contained", "<u4"), ("depth_min", "<u4"), ("depth_max", "<u4"), ("reserved", "<u4"),
+                           ("length", "<u8"), ("start", "<u8"), ("read_count", "<u8"), ("depth_sum", "<u8"), ("depth_sq_sum", "<u8")])
+assert CEDGE_DTYPE.itemsize == 40 and CITEM_DTYPE.itemsize == 8 and UNITIG_DTYPE.itemsize == 32 and COVERAGE_DTYPE.itemsize == 64
 assert EDGE_DTYPE.itemsize == C.sizeof(Edge) == 12
 
 
@@ -273,6 +276,35 @@ class OverlapGraph:
         """Spells the (canonical) unitigs and writes them as FASTA (ogb_graph_write_unitigs); returns the spell stats."""
         st = self.spell(canonical)
         check(lib().ogb_graph_write_unitigs(self.ctx._h, str(path).encode()))
+        return st
+
+    def coverage(self, canonical=True, first=0, count=None):
+        """Spells unitigs [first, first + count) (see spell) and computes their per-base read depth on the device, weighted by the
+        Dataset's read frequencies, contained reads placed inside their super reads (ogb_graph_coverage). Returns (records as
+        COVERAGE_DTYPE in the unitig order, the ogb_coverage_stats as a dict)."""
+        from ._lib import CoverageStats
+        self.spell(canonical, first, count)
+        freq = np.ascontiguousarray(self.dataSet.frequencies(), dtype=np.uint32)
+        st = CoverageStats()
+        check(lib().ogb_graph_coverage(self.ctx._h, freq.ctypes.data, len(freq), C.byref(st)))
+        recs = np.zeros(st.unitigs, dtype=COVERAGE_DTYPE)
+        check(lib().ogb_graph_unitig_coverage(self.ctx._h, recs.ctypes.data, len(recs), None, 0))
+        return recs, st.as_dict()
+
+    def depth(self, canonical=True, first=0, count=None):
+        """(records, depth): as coverage(), plus the uint32 per-base depth in the spell's word-aligned layout -- unitig i is
+        depth[start : start + length], the bases up to its next multiple of 32 are 0."""
+        recs, _ = self.coverage(canonical, first, count)
+        words = int((recs["start"][-1] + recs["length"][-1] + 31) // 32) if len(recs) else 0     # the layout ends with the last unitig
+        out = np.zeros(32 * words, dtype=np.uint32)
+        check(lib().ogb_graph_unitig_coverage(self.ctx._h, recs.ctypes.data, len(recs), out.ctypes.data, len(out)))
+        return recs, out
+
+    def write_coverage(self, path, canonical=True):
+        """Computes the coverage of the (canonical) unitigs and writes it as TSV (ogb_graph_write_coverage), one line per unitig
+        named as in write_unitigs' FASTA; returns the coverage stats."""
+        _, st = self.coverage(canonical)
+        check(lib().ogb_graph_write_coverage(self.ctx._h, str(path).encode()))
         return st
 
     def checksum(self, pre=False):

@@ -12,9 +12,11 @@
 #include "ogb_kernels.cuh"
 #include "ogb_contract.cuh"
 #include "ogb_spell.cuh"
+#include "ogb_coverage.cuh"
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <dlfcn.h>
@@ -108,7 +110,7 @@ template <class T> struct Tmp {
 	void release() { if (p) cudaFreeAsync(p, st); p = nullptr; }
 };
 
-enum { EV_BEGIN = 0, EV_PACK0, EV_PACK1, EV_HASH0, EV_HASH1, EV_CONT0, EV_CONT1, EV_OVL0, EV_OVL1, EV_XPRE1, EV_MARK1, EV_RED1, EV_K3A, EV_K3B, EV_T0, EV_T1, EV_COUNT };
+enum { EV_BEGIN = 0, EV_PACK0, EV_PACK1, EV_HASH0, EV_HASH1, EV_CONT0, EV_CONT1, EV_OVL0, EV_OVL1, EV_XPRE1, EV_MARK1, EV_RED1, EV_K3A, EV_K3B, EV_T0, EV_T1, EV_CV1, EV_CV2, EV_COUNT };
 
 struct ogb_context {
 	int device = 0, rank = 0, nranks = 1, sm_count = 148;
@@ -202,6 +204,12 @@ struct ogb_context {
 	bool have_spelled = false;
 	u64 sp_first = 0;
 	ogb_spell_stats spst = {};
+	// unitig coverage (ogb_coverage.cuh): contained-read offsets and CSR, placement scan, difference array (then the profile), its scan
+	Pool<u32> cv_freq, cv_q, cv_cnt, cv_clist, cv_np, cv_depth;
+	Pool<u64> cv_cstart, cv_ppos, cv_scan;
+	Pool<ogb_unitig_coverage> cv_rec;
+	bool have_covered = false;
+	ogb_coverage_stats cvst = {};
 	// L2 persistence window on the bucket summary (l2_keep_summary)
 	const void *l2_window_ptr = nullptr;
 	size_t l2_window_bytes = 0;
@@ -378,6 +386,8 @@ extern "C" void ogb_context_destroy(ogb_context *c)
 	c->s_state.release(); c->s_ready.release(); c->s_flag.release(); c->s_epos.release(); c->s_lpos.release(); c->s_ctr.release(); c->s_out.release(); c->s_out_items.release();
 	c->sp_sel.release(); c->sp_ioff.release(); c->sp_nw.release(); c->sp_rank.release(); c->sp_ipos.release(); c->sp_wpos.release(); c->sp_words.release();
 	c->sp_rec.release(); c->sp_ascii.release();
+	c->cv_freq.release(); c->cv_q.release(); c->cv_cnt.release(); c->cv_clist.release(); c->cv_np.release(); c->cv_depth.release();
+	c->cv_cstart.release(); c->cv_ppos.release(); c->cv_scan.release(); c->cv_rec.release();
 	if (c->d_ctr) cudaFree(c->d_ctr);
 	if (c->d_tot) cudaFree(c->d_tot);
 	if (c->d_cursor) cudaFree(c->d_cursor);
@@ -457,7 +467,7 @@ static int upload_common(ogb_context *c, u64 total_words, const std::vector<u64>
 	}
 	c->slot_cap = 64;
 	c->reads_stamp++;
-	c->have_reads = true; c->have_table = false; c->contain_done = false; c->any_contained = false; c->have_graph = false; c->have_pre = false; c->have_spelled = false;
+	c->have_reads = true; c->have_table = false; c->contain_done = false; c->any_contained = false; c->have_graph = false; c->have_pre = false; c->have_spelled = false; c->have_covered = false;
 	return OGB_OK;
 }
 
@@ -1410,7 +1420,7 @@ extern "C" int ogb_build_graph(ogb_context *c, int keep_pre)
 	OGB_TRY(l2_keep_summary(c, true));                                      // (a second build on the same index: the first one closed the window)
 	// buildOverlapGraphFromHashTable always marks contained reads first (OverlapGraph.cpp:140)
 	if (!c->contain_done) OGB_TRY(ogb_mark_contained(c));
-	c->have_graph = false; c->have_pre = false; c->have_simplified = false; c->have_spelled = false; c->n_final = 0; c->n_pre = 0;
+	c->have_graph = false; c->have_pre = false; c->have_simplified = false; c->have_spelled = false; c->have_covered = false; c->n_final = 0; c->n_pre = 0;
 	const u32 n = c->n;
 	if (n == 0) { c->have_graph = true; c->have_pre = keep_pre != 0; c->st.edges_pre = c->st.edges_pre_local = c->st.edges_final = c->st.nodes_final = 0; return OGB_OK; }
 	u32 lo, hi;
@@ -1751,7 +1761,7 @@ extern "C" int ogb_graph_simplify(ogb_context *c, ogb_simplify_stats *stats)
 	const u64 ne = c->n_final;
 	const u32 n = c->n;
 	if (ne >= (1ull << 31) || n >= (1u << 30)) { ogb_set_error("ogb_graph_simplify: %llu edges / %u reads exceed the 31-bit entry and record indices", (unsigned long long)ne, n); return OGB_E_CAPACITY; }
-	c->have_simplified = false; c->have_spelled = false;
+	c->have_simplified = false; c->have_spelled = false; c->have_covered = false;
 	ogb_simplify_stats st = {};
 	st.n_edges_in = ne;
 	const u64 nrec = 2 * ((u64)n + 1);
@@ -1902,7 +1912,7 @@ extern "C" int ogb_graph_spell(ogb_context *c, int canonical_only, uint64_t firs
 	if (!c) { ogb_set_error("ogb_graph_spell: NULL context"); return OGB_E_ARG; }
 	if (!c->have_simplified || c->s_stamp != c->reads_stamp) { ogb_set_error("ogb_graph_spell: run ogb_graph_simplify on the uploaded reads first"); return OGB_E_STATE; }
 	CUDA_TRY(cudaSetDevice(c->device));
-	c->have_spelled = false;
+	c->have_spelled = false; c->have_covered = false;
 	const u64 ne = c->sst.n_edges_out, ni = c->sst.n_items, cap = std::min<u64>(count, ne);
 	ogb_spell_stats st = {};
 	const int grid_max = c->sm_count * 8;
@@ -2035,6 +2045,115 @@ extern "C" int ogb_graph_write_unitigs(ogb_context *c, const char *path)
 	if (stage) cudaFreeHost(stage);
 	if (fclose(f) != 0 && rc == OGB_OK) { ogb_set_error("ogb_graph_write_unitigs: closing %s failed", path); rc = OGB_E_IO; }
 	return rc;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Unitig coverage: see ogb_coverage.cuh.
+// ------------------------------------------------------------------------------------------------
+extern "C" int ogb_graph_coverage(ogb_context *c, const uint32_t *freq, uint64_t n, ogb_coverage_stats *stats)
+{
+	if (!c) { ogb_set_error("ogb_graph_coverage: NULL context"); return OGB_E_ARG; }
+	if (!c->have_spelled) { ogb_set_error("ogb_graph_coverage: run ogb_graph_spell on the uploaded reads first"); return OGB_E_STATE; }
+	if (n != c->n || (n && !freq)) { ogb_set_error("ogb_graph_coverage: need the frequencies of the %u uploaded reads (got %llu)", c->n, (unsigned long long)(freq ? n : 0)); return OGB_E_ARG; }
+	const u64 nu = c->spst.unitigs, nw = c->spst.words, nb = 32 * nw + 1, ni = c->sst.n_items;
+	if (nb >= (1ull << 32)) { ogb_set_error("ogb_graph_coverage: %llu bases of layout exceed the 32-bit scan", (unsigned long long)nb); return OGB_E_CAPACITY; }
+	CUDA_TRY(cudaSetDevice(c->device));
+	c->have_covered = false;
+	const u32 nr = c->n;
+	const bool locate = c->any_contained && nr;
+	ogb_coverage_stats st = {};
+	st.unitigs = nu; st.bases = c->spst.bases;
+	const int grid_max = c->sm_count * 8;
+	auto grid = [&](u64 items) { return (unsigned)std::max<u64>(1, std::min<u64>((items + 255) / 256, (u64)grid_max)); };
+	OGB_TRY(c->cv_freq.ensure(std::max<u32>(nr, 1))); OGB_TRY(c->cv_rec.ensure(std::max<u64>(nu, 1))); OGB_TRY(c->cv_np.ensure(std::max<u64>(nu, 1)));
+	OGB_TRY(c->cv_ppos.ensure(nu + 1)); OGB_TRY(c->cv_depth.ensure(nb)); OGB_TRY(c->cv_scan.ensure(nb)); OGB_TRY(c->s_ctr.ensure(16));
+	if (locate) { OGB_TRY(c->cv_q.ensure(nr)); OGB_TRY(c->cv_cnt.ensure(nr)); OGB_TRY(c->cv_cstart.ensure((u64)nr + 1)); OGB_TRY(c->cv_clist.ensure(nr)); }
+	u64 *ctr = c->s_ctr.p;                                                        // [0] unplaced, [1] contained placements, [2] scan total
+	CovArgs A;
+	A.S = spell_args(c); A.ppos = c->cv_ppos.p; A.freq = c->cv_freq.p;
+	A.sup = locate ? c->sup.p : nullptr; A.q = locate ? c->cv_q.p : nullptr; A.cstart = locate ? c->cv_cstart.p : nullptr; A.clist = locate ? c->cv_clist.p : nullptr;
+	CUDA_TRY(cudaEventRecord(c->ev[EV_T0], c->stream));
+	CUDA_TRY(cudaMemsetAsync(ctr, 0, 3 * sizeof(u64), c->stream));
+	if (nr) CUDA_TRY(cudaMemcpyAsync(c->cv_freq.p, freq, (size_t)nr * sizeof(u32), cudaMemcpyHostToDevice, c->stream));
+	if (locate) {
+		CUDA_TRY(cudaMemsetAsync(c->cv_cnt.p, 0, (size_t)nr * sizeof(u32), c->stream));
+		k_cov_locate<<<grid(nr), 256, 0, c->stream>>>(A, nr, c->cv_q.p, c->cv_cnt.p, ctr);
+		OGB_TRY(exclusive_scan(c, c->cv_cnt.p, nr, c->cv_cstart.p, c->cv_cstart.p + nr, nullptr, nullptr));
+		CUDA_TRY(cudaMemsetAsync(c->cv_cnt.p, 0, (size_t)nr * sizeof(u32), c->stream));          // now the fill cursors
+		k_cov_scatter<<<grid(nr), 256, 0, c->stream>>>(c->sup.p, c->cv_q.p, nr, c->cv_cstart.p, c->cv_cnt.p, c->cv_clist.p);
+		st.launches += 5;
+	}
+	CUDA_TRY(cudaEventRecord(c->ev[EV_CV1], c->stream));
+	CUDA_TRY(cudaMemsetAsync(c->cv_depth.p, 0, nb * sizeof(u32), c->stream));   // the difference array until the scan
+	CUDA_TRY(cudaMemsetAsync(c->cv_ppos.p + nu, 0, sizeof(u64), c->stream));
+	if (nu) {
+		k_cov_init<<<grid(nu), 256, 0, c->stream>>>(c->sp_rec.p, c->s_out.p, nu, c->cv_rec.p, c->cv_np.p);
+		OGB_TRY(exclusive_scan(c, c->cv_np.p, (u32)nu, c->cv_ppos.p, c->cv_ppos.p + nu, nullptr, nullptr));
+		k_cov_place<<<grid(ni + 2 * nu), 256, 0, c->stream>>>(A, c->cv_ppos.p + nu, c->cv_depth.p, c->cv_rec.p, ctr + 1);
+		OGB_TRY(exclusive_scan(c, c->cv_depth.p, (u32)nb, c->cv_scan.p, ctr + 2, nullptr, nullptr));
+		st.launches += 8;
+	}
+	CUDA_TRY(cudaEventRecord(c->ev[EV_CV2], c->stream));
+	if (nw) {
+		k_cov_reduce<<<grid(nw), 256, 0, c->stream>>>(c->cv_scan.p, c->sp_wpos.p, nu, nw, c->cv_depth.p, c->cv_rec.p);
+		st.launches++;
+	}
+	CUDA_TRY(cudaGetLastError());
+	CUDA_TRY(cudaEventRecord(c->ev[EV_T1], c->stream));
+	u64 h[3] = {0, 0, 0};
+	CUDA_TRY(cudaMemcpyAsync(h, ctr, 2 * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(h + 2, c->cv_ppos.p + nu, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaStreamSynchronize(c->stream));
+	st.unplaced = h[0]; st.contained_placements = h[1]; st.placements = h[2];
+	st.ms = ev_ms(c, EV_T0, EV_T1); st.ms_locate = ev_ms(c, EV_T0, EV_CV1); st.ms_depth = ev_ms(c, EV_CV1, EV_CV2); st.ms_reduce = ev_ms(c, EV_CV2, EV_T1);
+	c->cvst = st;
+	c->have_covered = true;
+	if (stats) *stats = st;
+	return OGB_OK;
+}
+
+extern "C" int ogb_graph_unitig_coverage(ogb_context *c, ogb_unitig_coverage *recs, uint64_t rec_cap, uint32_t *depth, uint64_t depth_cap)
+{
+	if (!c) { ogb_set_error("ogb_graph_unitig_coverage: NULL context"); return OGB_E_ARG; }
+	if (!c->have_covered) { ogb_set_error("ogb_graph_unitig_coverage: run ogb_graph_coverage first"); return OGB_E_STATE; }
+	const u64 nu = c->cvst.unitigs, nd = 32 * c->spst.words;
+	if ((nu && (!recs || rec_cap < nu)) || (depth && depth_cap < nd)) {
+		ogb_set_error("ogb_graph_unitig_coverage: need room for %llu records and %llu depth entries", (unsigned long long)nu, (unsigned long long)nd);
+		return OGB_E_CAPACITY;
+	}
+	CUDA_TRY(cudaSetDevice(c->device));
+	if (nu) CUDA_TRY(cudaMemcpyAsync(recs, c->cv_rec.p, nu * sizeof(ogb_unitig_coverage), cudaMemcpyDeviceToHost, c->stream));
+	if (depth && nd) CUDA_TRY(cudaMemcpyAsync(depth, c->cv_depth.p, nd * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaStreamSynchronize(c->stream));
+	return OGB_OK;
+}
+
+extern "C" int ogb_graph_write_coverage(ogb_context *c, const char *path)
+{
+	if (!c || !path) { ogb_set_error("ogb_graph_write_coverage: NULL argument"); return OGB_E_ARG; }
+	if (!c->have_covered) { ogb_set_error("ogb_graph_write_coverage: run ogb_graph_coverage first"); return OGB_E_STATE; }
+	CUDA_TRY(cudaSetDevice(c->device));
+	const u64 nu = c->cvst.unitigs;
+	std::vector<ogb_unitig_coverage> cov(nu);
+	std::vector<ogb_unitig> rec(nu);                                           // src, dst
+	if (nu) {
+		CUDA_TRY(cudaMemcpyAsync(cov.data(), c->cv_rec.p, nu * sizeof(ogb_unitig_coverage), cudaMemcpyDeviceToHost, c->stream));
+		CUDA_TRY(cudaMemcpyAsync(rec.data(), c->sp_rec.p, nu * sizeof(ogb_unitig), cudaMemcpyDeviceToHost, c->stream));
+		CUDA_TRY(cudaStreamSynchronize(c->stream));
+	}
+	FILE *f = fopen(path, "wb");
+	if (!f) { ogb_set_error("ogb_graph_write_coverage: cannot open %s for writing", path); return OGB_E_IO; }
+	fprintf(f, "#name\tsrc\tdst\tlength\treads\tcontained\tread_count\tmean_depth\tsd_depth\tmin_depth\tmax_depth\n");
+	for (u64 r = 0; r < nu; r++) {
+		const ogb_unitig_coverage &v = cov[r];
+		const double len = (double)v.length, mean = (double)v.depth_sum / len;
+		const double sd = std::sqrt(std::max(0.0, (double)v.depth_sq_sum / len - mean * mean));
+		fprintf(f, "unitig_%llu\t%u\t%u\t%llu\t%u\t%u\t%llu\t%.4f\t%.4f\t%u\t%u\n", (unsigned long long)(c->sp_first + r), rec[r].src, rec[r].dst,
+		        (unsigned long long)v.length, v.reads, v.contained, (unsigned long long)v.read_count, mean, sd, v.depth_min, v.depth_max);
+	}
+	if (ferror(f)) { fclose(f); ogb_set_error("ogb_graph_write_coverage: write to %s failed", path); return OGB_E_IO; }
+	if (fclose(f) != 0) { ogb_set_error("ogb_graph_write_coverage: closing %s failed", path); return OGB_E_IO; }
+	return OGB_OK;
 }
 
 extern "C" int ogb_get_stats(ogb_context *c, ogb_stats *out)

@@ -16,6 +16,7 @@ OverlapGraph::OverlapGraph(void)
 	memset(&lastStats, 0, sizeof lastStats);
 	memset(&lastSimplifyStats, 0, sizeof lastSimplifyStats);
 	memset(&lastSpellStats, 0, sizeof lastSpellStats);
+	memset(&lastCoverageStats, 0, sizeof lastCoverageStats);
 }
 
 OverlapGraph::OverlapGraph(HashTable *ht)
@@ -24,6 +25,7 @@ OverlapGraph::OverlapGraph(HashTable *ht)
 	memset(&lastStats, 0, sizeof lastStats);
 	memset(&lastSimplifyStats, 0, sizeof lastSimplifyStats);
 	memset(&lastSpellStats, 0, sizeof lastSpellStats);
+	memset(&lastCoverageStats, 0, sizeof lastCoverageStats);
 	buildOverlapGraphFromHashTable(ht);
 }
 
@@ -118,6 +120,19 @@ bool OverlapGraph::simplifyGraph(void)
 	}
 	delete hashTable;														// :210 -- the graph owns and frees the table
 	hashTable = NULL;
+	return true;
+}
+
+// Per-base read depth of the unitigs simplifyGraph() spelled (spellInBuild), weighted by the Dataset's read frequencies and with the
+// contained reads placed in their super reads, written as TSV (ogb_graph_write_coverage). The device context stays: call it before
+// saveUnitigsToFile, which releases it.
+bool OverlapGraph::saveUnitigCoverageToFile(string fileName)
+{
+	if (!hashTable) throw OgbFailure(OGB_E_STATE, "saveUnitigCoverageToFile: no unitigs on the device (set OverlapGraph::spellInBuild before the build)");
+	ogb_context *ctx = hashTable->getContext();
+	const uint64_t n = dataSet->getNumberOfUniqueReads();
+	ogbCheck(ogb_graph_coverage(ctx, ogb_dataset_frequencies(dataSet->handle()), n, &lastCoverageStats), "OverlapGraph::saveUnitigCoverageToFile");
+	ogbCheck(ogb_graph_write_coverage(ctx, fileName.c_str()), "OverlapGraph::saveUnitigCoverageToFile");
 	return true;
 }
 

@@ -41,6 +41,7 @@ class OverlapGraph
 		void clearGraph(void);
 		ogb_simplify_stats lastSimplifyStats;
 		ogb_spell_stats lastSpellStats;
+		ogb_coverage_stats lastCoverageStats;
 
 	public:
 		bool flowComputed;
@@ -65,6 +66,7 @@ class OverlapGraph
 		bool setDataset(Dataset *dataset) { dataSet = dataset; dataset->readMatePairsFromFile(); return true; }
 		void sortEdges();
 		bool saveGraphToFile(string fileName);			// OverlapGraph.cpp:1219-1259: the reference's .unitig text format
+		bool saveUnitigCoverageToFile(string fileName);	// per-base read depth of the spelled unitigs as TSV (ogb_graph_coverage); before saveUnitigsToFile
 		bool saveUnitigsToFile(string fileName);		// the unitigs spelled in the build as FASTA (ogb_graph_write_unitigs); frees the hash table
 		bool readGraphFromFile(string fileName);		// OverlapGraph.cpp:1267-1367 (resume path, main.cpp:36-42)
 		Edge *findEdge(UINT64 source, UINT64 destination);
@@ -73,6 +75,7 @@ class OverlapGraph
 		const ogb_stats &getBuildStats(void) const { return lastStats; }
 		const ogb_simplify_stats &getSimplifyStats(void) const { return lastSimplifyStats; }
 		const ogb_spell_stats &getSpellStats(void) const { return lastSpellStats; }
+		const ogb_coverage_stats &getCoverageStats(void) const { return lastCoverageStats; }
 };
 
 #endif

@@ -4,11 +4,12 @@
 // (calculateFlow, the three simplification loops, printGraph) is host code that consumes the graph
 // this program produces and is not part of this library.
 //
-//   ogb_overlap -l minOverlap [-se n files...] [-pe n files...] [-f prefix] [--dump file] [--unitigs file]
+//   ogb_overlap -l minOverlap [-se n files...] [-pe n files...] [-f prefix] [--dump file] [--unitigs file] [--coverage file]
 //
 // --dump writes the graph in the binary format the parity tests read, so one comparator reads
 // the output of the unmodified reference and of this program. --unitigs writes the sequences of the canonical unitigs of the
-// simplified graph as FASTA, spelled on the device (OverlapGraph::spellInBuild, saveUnitigsToFile).
+// simplified graph as FASTA, spelled on the device (OverlapGraph::spellInBuild, saveUnitigsToFile). --coverage writes their per-base
+// read depth summary as TSV, contained reads included (saveUnitigCoverageToFile); the names join with the FASTA's.
 #include "Common.h"
 #include "Dataset.h"
 #include "Edge.h"
@@ -81,7 +82,7 @@ int main(int argc, char **argv)
 	UINT64 minimumOverlapLength = 0;
 	vector<string> pairedEndFileNames, singleEndFileNames;
 	string allFileName = "";
-	const char *dumpPath = NULL, *resavePath = NULL, *matesPath = NULL, *unitigsPath = NULL;
+	const char *dumpPath = NULL, *resavePath = NULL, *matesPath = NULL, *unitigsPath = NULL, *coveragePath = NULL;
 	bool startFromUnitigGraph = false;
 	for (int i = 1; i < argc; i++) {
 		string a = argv[i];
@@ -95,8 +96,9 @@ int main(int argc, char **argv)
 		else if (a == "--resave" && i + 1 < argc) resavePath = argv[++i];
 		else if (a == "--mates" && i + 1 < argc) matesPath = argv[++i];
 		else if (a == "--unitigs" && i + 1 < argc) unitigsPath = argv[++i];
+		else if (a == "--coverage" && i + 1 < argc) coveragePath = argv[++i];
 		else {
-			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file] [--unitigs file]" << endl;
+			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file] [--unitigs file] [--coverage file]" << endl;
 			return a == "-h" || a == "--help" ? 0 : 1;
 		}
 	}
@@ -106,6 +108,10 @@ int main(int argc, char **argv)
 	}
 	if (startFromUnitigGraph && unitigsPath) {
 		cerr << "ogb_overlap: --unitigs needs the build on the device; -s resumes from a .unitig file without one" << endl;
+		return 1;
+	}
+	if (startFromUnitigGraph && coveragePath) {
+		cerr << "ogb_overlap: --coverage needs the build on the device; -s resumes from a .unitig file without one" << endl;
 		return 1;
 	}
 	try {
@@ -125,7 +131,7 @@ int main(int argc, char **argv)
 			return 0;
 		}
 		if (dumpPath) OverlapGraph::simplifyInBuild = false;											// --dump wants the graph as it is at OverlapGraph.cpp:210
-		if (unitigsPath) OverlapGraph::spellInBuild = true;
+		if (unitigsPath || coveragePath) OverlapGraph::spellInBuild = true;
 		HashTable *hashTable = new HashTable();															// main.cpp:45
 		hashTable->insertDataset(dataSet, minimumOverlapLength);										// main.cpp:46
 		overlapGraph = new OverlapGraph(hashTable); //hashTable deleted by this function after building the graph (main.cpp:47)
@@ -143,6 +149,12 @@ int main(int argc, char **argv)
 		     << " nodes: " << overlapGraph->getNumberOfNodes() << " edges: " << overlapGraph->getNumberOfEdges()
 		     << " device ms: " << st.ms_total << " + simplification " << ss.ms << " (" << ss.merges << " merges, " << ss.dead_ends << " dead ends, "
 		     << ss.iterations << " iterations, " << ss.rounds << " rounds)" << endl;
+		if (coveragePath) {
+			overlapGraph->saveUnitigCoverageToFile(coveragePath);
+			const ogb_coverage_stats &cv = overlapGraph->getCoverageStats();
+			cout << "coverage: " << cv.unitigs << " unitigs " << cv.bases << " bases " << cv.placements << " placements " << cv.contained_placements
+			     << " contained placements " << cv.unplaced << " unplaced, coverage device ms: " << cv.ms << " (" << coveragePath << ")" << endl;
+		}
 		if (unitigsPath) {
 			overlapGraph->saveUnitigsToFile(unitigsPath);
 			const ogb_spell_stats &sp = overlapGraph->getSpellStats();
