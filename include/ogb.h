@@ -173,6 +173,11 @@ int ogb_dataset_get_read(const ogb_dataset *ds, uint64_t id, int strand, char *o
  * the string is not in the dataset (the reference exits there). */
 int ogb_dataset_find_read(const ogb_dataset *ds, const char *bases, uint32_t len, uint64_t *id);
 
+/* The reads added to a data set that is not finalized, as added (no filter, no case folding): read i = (*bases)[(*offsets)[i] ..
+ * (*offsets)[i+1]), *n reads. Views into the data set, valid until it changes. A finalized data set: OGB_E_STATE. Lets a caller read
+ * sample files (ogb_dataset_add_file) for ogb_graph_map_reads. */
+int ogb_dataset_raw_reads(const ogb_dataset *ds, const char **bases, const uint64_t **offsets, uint64_t *n);
+
 /* ----------------------------------------------------------------------------------------------
  * Device side.
  * -------------------------------------------------------------------------------------------- */
@@ -399,6 +404,56 @@ int ogb_graph_unitig_coverage(ogb_context *ctx, ogb_unitig_coverage *recs, uint6
  * with i as in ogb_graph_write_unitigs (the names join with the FASTA), mean = depth_sum / length and
  * sd = sqrt(max(0, depth_sq_sum / length - mean^2)) in double, printed %.4f. OGB_E_IO when the file cannot be written. */
 int ogb_graph_write_coverage(ogb_context *ctx, const char *path);
+
+/* ----------------------------------------------------------------------------------------------
+ * Sample mapping: per-sample read depth of the unitigs of the last ogb_graph_spell, on the device (csrc/ogb_map.cuh), for the
+ * contig x sample depth tables metagenome binners take. A sample is a list of ASCII reads. A read is kept iff it passes the Dataset
+ * filter for the build's minOverlap m (length > m and < 65536, ACGT only in either case, no base count >= (UINT64)(len*.8)). A
+ * placement of a kept read s of length L is (u, p) with bases [p, p + L) of unitig u equal to s or to its reverse complement; a
+ * read equal to its own reverse complement is tested on one strand only. Every placement adds 1 to the depth on [p, p + L). Raw reads
+ * count one by one, and a read with several placements counts at each. Reads with errors or clipped alignments do not map.
+ * -------------------------------------------------------------------------------------------- */
+
+#define OGB_MAP_FILTERED 0xFFFFFFFFu /* hits[i] of a read the filter dropped */
+
+typedef struct ogb_map_stats {
+	uint64_t reads_in;
+	uint64_t filtered;
+	uint64_t mapped;          /* kept reads with >= 1 placement */
+	uint64_t multi;           /* kept reads with >= 2 placements */
+	uint64_t placements;
+	uint64_t index_entries;   /* positions of the K-mer index over the unitigs, K = min(32, m + 1) */
+	uint64_t index_buckets;
+	uint32_t sample;          /* this sample's index among the samples mapped since the spell */
+	uint32_t launches;
+	float ms;                 /* device time of ogb_graph_map_reads = the four parts below */
+	float ms_index;           /* index build; 0 when the index of an earlier sample was reused */
+	float ms_upload;          /* reads to the device, filter, packing */
+	float ms_map;             /* lookups, verification, difference array (and the hit counts to the host) */
+	float ms_reduce;          /* scan, per-base profile and per-unitig sums */
+	uint32_t reserved;
+} ogb_map_stats; /* 88 bytes */
+
+/* Maps one sample: n reads, read i = bases[offsets[i] .. offsets[i+1]) (ASCII), onto the unitigs of the last ogb_graph_spell (the
+ * same range and selection), in bounded chunks of reads. Its records (ogb_unitig_coverage, one per unitig: reads = read_count = its
+ * placements, contained = 0, depth sums, min and max as in ogb_graph_coverage) are appended to those of the samples mapped since the
+ * spell, 64 B x unitigs per sample on the host; its u32 profile stays on the device until the next sample. hits (NULL or n entries):
+ * the placements of every read, OGB_MAP_FILTERED for a read the filter dropped. The K-mer index is built by the first mapping after a
+ * spell and kept for the later samples. n = 0 is a valid sample. No spell on the current reads: OGB_E_STATE; a layout of >= 2^32
+ * bases: OGB_E_CAPACITY; NULL buffers with n > 0 or offsets that decrease: OGB_E_ARG. Integers only: two runs give the same bits.
+ * An upload, build, simplify or spell drops the index and the samples. The coverage of ogb_graph_coverage is left as it is. */
+int ogb_graph_map_reads(ogb_context *ctx, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t *hits, ogb_map_stats *stats);
+/* Copies the records of sample `sample` (rec_cap >= unitigs) and, when depth is not NULL, its u32 profile in the spell's word-aligned
+ * layout (depth_cap >= 32 * ogb_spell_stats.words) -- kept for the last sample only: depth must be NULL for any other. No samples:
+ * OGB_E_STATE; a sample beyond the last, or depth for an earlier one: OGB_E_ARG; OGB_E_CAPACITY names the sizes needed. */
+int ogb_graph_sample_coverage(ogb_context *ctx, uint32_t sample, ogb_unitig_coverage *recs, uint64_t rec_cap, uint32_t *depth, uint64_t depth_cap);
+/* Writes the depth table of every sample since the spell in MetaBAT's layout (jgi_summarize_bam_contig_depths):
+ *     contigName  contigLen  totalAvgDepth  <name_1>  <name_1>-var  ...
+ * then per unitig, tab-separated: unitig_<i> (i as in ogb_graph_write_unitigs), its length, the sum of the means, and per sample the
+ * mean depth_sum / length and the population variance max(0, depth_sq_sum / length - mean^2), in double, printed %.4f. No edge
+ * trimming. names: one per sample (NULL: sample_<j>). No samples: OGB_E_STATE; a name with a tab or a newline: OGB_E_ARG; a file that
+ * cannot be written: OGB_E_IO. */
+int ogb_graph_write_depths(ogb_context *ctx, const char *path, const char *const *names);
 
 int ogb_get_stats(ogb_context *ctx, ogb_stats *out);
 

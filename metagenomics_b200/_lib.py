@@ -66,6 +66,18 @@ class CoverageStats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_ if n != "reserved"}
 
 
+class MapStats(C.Structure):
+    """ogb_map_stats (include/ogb.h)."""
+    _fields_ = [(n, C.c_uint64) for n in ("reads_in", "filtered", "mapped", "multi", "placements", "index_entries", "index_buckets")] + [
+        (n, C.c_uint32) for n in ("sample", "launches")] + [(n, C.c_float) for n in ("ms", "ms_index", "ms_upload", "ms_map", "ms_reduce")] + [
+        ("reserved", C.c_uint32)]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_ if n != "reserved"}
+
+
+OGB_MAP_FILTERED = 0xFFFFFFFF
+
 # every symbol include/ogb.h declares: name -> (restype, argtypes)
 _u64p = C.POINTER(C.c_uint64)
 _vp = C.c_void_p
@@ -89,6 +101,7 @@ PROTOTYPES = {
     "ogb_dataset_frequencies": (_vp, [_vp]),
     "ogb_dataset_get_read": (C.c_int, [_vp, C.c_uint64, C.c_int, _vp, C.c_uint32, C.POINTER(C.c_uint32)]),
     "ogb_dataset_find_read": (C.c_int, [_vp, C.c_char_p, C.c_uint32, _u64p]),
+    "ogb_dataset_raw_reads": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_vp), _u64p]),
     "ogb_context_create": (C.c_int, [C.POINTER(_vp), C.c_int]),
     "ogb_nccl_unique_id": (C.c_int, [_vp]),
     "ogb_context_create_dist": (C.c_int, [C.POINTER(_vp), C.c_int, C.c_int, C.c_int, _vp]),
@@ -118,6 +131,9 @@ PROTOTYPES = {
     "ogb_graph_coverage": (C.c_int, [_vp, _vp, C.c_uint64, C.POINTER(CoverageStats)]),
     "ogb_graph_unitig_coverage": (C.c_int, [_vp, _vp, C.c_uint64, _vp, C.c_uint64]),
     "ogb_graph_write_coverage": (C.c_int, [_vp, C.c_char_p]),
+    "ogb_graph_map_reads": (C.c_int, [_vp, _vp, _vp, C.c_uint64, _vp, C.POINTER(MapStats)]),
+    "ogb_graph_sample_coverage": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint64, _vp, C.c_uint64]),
+    "ogb_graph_write_depths": (C.c_int, [_vp, C.c_char_p, _vp]),
     "ogb_get_stats": (C.c_int, [_vp, C.POINTER(Stats)]),
     "ogb_timer_begin": (C.c_int, [_vp]),
     "ogb_timer_end": (C.c_int, [_vp, C.POINTER(C.c_float)]),

@@ -260,6 +260,7 @@ class OverlapGraph:
         from ._lib import SpellStats
         st = SpellStats()
         check(lib().ogb_graph_spell(self.ctx._h, 1 if canonical else 0, int(first), 2**64 - 1 if count is None else int(count), C.byref(st)))
+        self._spelled, self._samples = st.as_dict(), 0             # a spell starts a new list of samples (map_reads)
         return st.as_dict()
 
     def unitigs(self, canonical=True, ascii=True, first=0, count=None):
@@ -306,6 +307,63 @@ class OverlapGraph:
         _, st = self.coverage(canonical)
         check(lib().ogb_graph_write_coverage(self.ctx._h, str(path).encode()))
         return st
+
+    def map_reads(self, reads=None, bases=None, offsets=None, hits=False):
+        """Maps one sample -- a list of str/bytes reads, or flat ASCII bases + offsets (n + 1) -- onto the unitigs of the last spell()
+        (ogb_graph_map_reads): every read that passes the Dataset filter counts 1 on every exact occurrence of itself or its reverse
+        complement. The sample is appended to the samples since that spell. Returns (records as COVERAGE_DTYPE in the unitig order:
+        reads = read_count = placements, the ogb_map_stats as a dict[, hits]): hits = uint32 placements per read, OGB_MAP_FILTERED
+        for a filtered read."""
+        if reads is not None:
+            bases, offsets = _reads_to_buffers(reads)
+        if bases is None:
+            bases, offsets = np.zeros(0, np.uint8), np.zeros(1, np.uint64)
+        bases = np.ascontiguousarray(bases, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        return self._map(bases.ctypes.data, offsets.ctypes.data, len(offsets) - 1, hits)
+
+    def map_file(self, path, hits=False):
+        """map_reads() of the reads of a FASTA or FASTQ file, read by the Dataset's parser (ogb_dataset_add_file)."""
+        ds = C.c_void_p()
+        check(lib().ogb_dataset_create(C.byref(ds)))
+        try:
+            check(lib().ogb_dataset_add_file(ds, str(path).encode()))
+            b, o, n = C.c_void_p(), C.c_void_p(), C.c_uint64()
+            check(lib().ogb_dataset_raw_reads(ds, C.byref(b), C.byref(o), C.byref(n)))
+            return self._map(b.value, o.value, n.value, hits)
+        finally:
+            lib().ogb_dataset_destroy(ds)
+
+    def _map(self, bases, offsets, n, hits):
+        from ._lib import MapStats
+        st = MapStats()
+        h = np.zeros(n, np.uint32) if hits else None
+        check(lib().ogb_graph_map_reads(self.ctx._h, bases, offsets, n, h.ctypes.data if hits else None, C.byref(st)))
+        self._samples = st.sample + 1
+        recs, _ = self.sample_depth(st.sample, profile=False)
+        return (recs, st.as_dict(), h) if hits else (recs, st.as_dict())
+
+    def sample_depth(self, sample=-1, profile=True):
+        """(records, profile) of a sample mapped since the last spell (-1: the last one): the profile is the uint32 per-base depth in
+        the spell's word-aligned layout (unitig i is profile[start : start + length]), kept for the last sample only -- None for
+        the others, or with profile=False."""
+        n = getattr(self, "_samples", 0)
+        j = n + sample if sample < 0 else sample
+        recs = np.zeros(self._spelled["unitigs"] if n else 0, dtype=COVERAGE_DTYPE)
+        depth = np.zeros(32 * self._spelled["words"], np.uint32) if n and profile and j == n - 1 else None
+        check(lib().ogb_graph_sample_coverage(self.ctx._h, max(j, 0), recs.ctypes.data, len(recs), None if depth is None else depth.ctypes.data,
+                                              0 if depth is None else len(depth)))
+        return recs, depth
+
+    def write_depths(self, path, names=None):
+        """Writes the depth table of every sample since the last spell in MetaBAT's layout (ogb_graph_write_depths); names: one per
+        sample (None: sample_<j>)."""
+        arr = None
+        if names is not None:
+            if len(names) != getattr(self, "_samples", 0):
+                raise ValueError(f"{len(names)} names for {getattr(self, '_samples', 0)} samples")
+            arr = (C.c_char_p * len(names))(*[str(x).encode() for x in names])
+        check(lib().ogb_graph_write_depths(self.ctx._h, str(path).encode(), arr))
 
     def checksum(self, pre=False):
         """[xor, sum] of the 64-bit mix of every edge tuple, computed on the device (the figure of tests/golden/full_size.json)."""

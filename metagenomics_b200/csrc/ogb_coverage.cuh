@@ -14,7 +14,8 @@
 //                  read's forward strand (cv_locate), counted per super read; an exclusive scan and k_cov_scatter build the CSR
 //                  super read -> contained reads. Skipped when no read is contained (one read length: K2 is a no-op).
 //   k_cov_init     thread per record: its ogb_unitig_coverage with zero sums, and its c + 2 placements; an exclusive scan gives the
-//                  flat placement index, and a binary search over it the record of a placement (as sp_word finds its unitig)
+//                  flat placement index, and a binary search over it the record of a placement (as sp_word finds its unitig). Without
+//                  nplace (sample mapping, ogb_map.cuh) the records start with reads = 0.
 //   k_cov_place    thread per placement (cv_place): +f at start + a, -f at start + a + L of a u32 difference array over the spell's
 //                  word-aligned layout (atomicAdd mod 2^32), for the read and for each contained read of it
 //   (scan)         one GLOBAL exclusive scan of the difference array: every +f/-f pair of a unitig lies in [start, start + length],
@@ -170,7 +171,8 @@ __global__ void __launch_bounds__(256) k_cov_init(const ogb_unitig *__restrict__
 		const ogb_unitig R = rec[u];
 		const cu32 c = edges[R.edge].count;
 		cv_record(R, out[u], c);
-		nplace[u] = c + 2;
+		if (nplace) nplace[u] = c + 2;
+		else out[u].reads = 0;                                 // sample mapping (ogb_map.cuh): reads counts its placements
 	}
 }
 // n_place on the device (the scan's total): no host round trip before the launch

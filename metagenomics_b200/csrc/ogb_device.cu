@@ -13,6 +13,7 @@
 #include "ogb_contract.cuh"
 #include "ogb_spell.cuh"
 #include "ogb_coverage.cuh"
+#include "ogb_map.cuh"
 
 #include <algorithm>
 #include <chrono>
@@ -110,7 +111,7 @@ template <class T> struct Tmp {
 	void release() { if (p) cudaFreeAsync(p, st); p = nullptr; }
 };
 
-enum { EV_BEGIN = 0, EV_PACK0, EV_PACK1, EV_HASH0, EV_HASH1, EV_CONT0, EV_CONT1, EV_OVL0, EV_OVL1, EV_XPRE1, EV_MARK1, EV_RED1, EV_K3A, EV_K3B, EV_T0, EV_T1, EV_CV1, EV_CV2, EV_COUNT };
+enum { EV_BEGIN = 0, EV_PACK0, EV_PACK1, EV_HASH0, EV_HASH1, EV_CONT0, EV_CONT1, EV_OVL0, EV_OVL1, EV_XPRE1, EV_MARK1, EV_RED1, EV_K3A, EV_K3B, EV_T0, EV_T1, EV_CV1, EV_CV2, EV_MP0, EV_MP1, EV_MP2, EV_MP3, EV_MP4, EV_COUNT };
 
 struct ogb_context {
 	int device = 0, rank = 0, nranks = 1, sm_count = 148;
@@ -210,6 +211,19 @@ struct ogb_context {
 	Pool<ogb_unitig_coverage> cv_rec;
 	bool have_covered = false;
 	ogb_coverage_stats cvst = {};
+	// sample mapping (ogb_map.cuh): K-mer index over the spell's layout, one chunk's reads, difference array (then the profile) and
+	// its scan; the records of every sample since the spell on the host
+	Pool<u32> mp_cnt, mp_good, mp_khits, mp_hits, mp_diff;
+	Pool<u64> mp_bstart, mp_ent, mp_roffs, mp_pos, mp_start, mp_meta, mp_words, mp_scan, mp_ctr;
+	Pool<char> mp_raw;
+	Pool<unsigned short> mp_len;
+	Pool<ogb_unitig_coverage> mp_rec;
+	bool mp_have_index = false;
+	u32 mp_K = 0;
+	u64 mp_buckets = 0, mp_entries = 0;
+	std::vector<ogb_unitig_coverage> mp_samples;   // spst.unitigs records per sample
+	u32 mp_n_samples = 0;
+	bool mp_have_profile = false;                    // mp_diff holds the profile of the last sample
 	// L2 persistence window on the bucket summary (l2_keep_summary)
 	const void *l2_window_ptr = nullptr;
 	size_t l2_window_bytes = 0;
@@ -388,6 +402,9 @@ extern "C" void ogb_context_destroy(ogb_context *c)
 	c->sp_rec.release(); c->sp_ascii.release();
 	c->cv_freq.release(); c->cv_q.release(); c->cv_cnt.release(); c->cv_clist.release(); c->cv_np.release(); c->cv_depth.release();
 	c->cv_cstart.release(); c->cv_ppos.release(); c->cv_scan.release(); c->cv_rec.release();
+	c->mp_cnt.release(); c->mp_good.release(); c->mp_khits.release(); c->mp_hits.release(); c->mp_diff.release(); c->mp_bstart.release(); c->mp_ent.release();
+	c->mp_roffs.release(); c->mp_pos.release(); c->mp_start.release(); c->mp_meta.release(); c->mp_words.release(); c->mp_scan.release(); c->mp_ctr.release();
+	c->mp_raw.release(); c->mp_len.release(); c->mp_rec.release();
 	if (c->d_ctr) cudaFree(c->d_ctr);
 	if (c->d_tot) cudaFree(c->d_tot);
 	if (c->d_cursor) cudaFree(c->d_cursor);
@@ -1913,6 +1930,7 @@ extern "C" int ogb_graph_spell(ogb_context *c, int canonical_only, uint64_t firs
 	if (!c->have_simplified || c->s_stamp != c->reads_stamp) { ogb_set_error("ogb_graph_spell: run ogb_graph_simplify on the uploaded reads first"); return OGB_E_STATE; }
 	CUDA_TRY(cudaSetDevice(c->device));
 	c->have_spelled = false; c->have_covered = false;
+	c->mp_have_index = false; c->mp_samples.clear(); c->mp_n_samples = 0; c->mp_have_profile = false;
 	const u64 ne = c->sst.n_edges_out, ni = c->sst.n_items, cap = std::min<u64>(count, ne);
 	ogb_spell_stats st = {};
 	const int grid_max = c->sm_count * 8;
@@ -1956,7 +1974,8 @@ extern "C" int ogb_graph_spell(ogb_context *c, int canonical_only, uint64_t firs
 	st.unitigs = std::min<u64>(cap, n_sel - first);
 	st.bases = h[1]; st.words = h[2];
 	c->spst = st;
-	OGB_TRY(c->sp_words.ensure(std::max<u64>(st.words, 1)));
+	OGB_TRY(c->sp_words.ensure(st.words + 1));                                    // + one zero word: sp_extract32 reads word w + 1 (ogb_map.cuh)
+	CUDA_TRY(cudaMemsetAsync(c->sp_words.p + st.words, 0, sizeof(u64), c->stream));
 	if (st.words) {
 		A = spell_args(c);
 		k_spell_words<<<grid(st.words), 256, 0, c->stream>>>(A, st.words, c->sp_rec.p, c->sp_words.p);
@@ -2153,6 +2172,194 @@ extern "C" int ogb_graph_write_coverage(ogb_context *c, const char *path)
 	}
 	if (ferror(f)) { fclose(f); ogb_set_error("ogb_graph_write_coverage: write to %s failed", path); return OGB_E_IO; }
 	if (fclose(f) != 0) { ogb_set_error("ogb_graph_write_coverage: closing %s failed", path); return OGB_E_IO; }
+	return OGB_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Sample mapping: see ogb_map.cuh.
+// ------------------------------------------------------------------------------------------------
+// Reads per chunk, and bytes per chunk (a bound for long reads): what the sample stage holds on the device at a time
+enum { OGB_MAP_CHUNK_READS = 1 << 22 };
+static const u64 OGB_MAP_CHUNK_BYTES = 1ull << 30;
+
+static MapArgs map_args(const ogb_context *c)
+{
+	MapArgs A;
+	A.layout = c->sp_words.p; A.wpos = c->sp_wpos.p; A.rec = c->sp_rec.p; A.n_rec = c->spst.unitigs;
+	A.K = c->mp_K; A.bmask = c->mp_buckets - 1; A.bstart = c->mp_bstart.p; A.ent = c->mp_ent.p;
+	A.rwords = c->mp_words.p; A.rmeta = c->mp_meta.p;
+	return A;
+}
+
+extern "C" int ogb_graph_map_reads(ogb_context *c, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t *hits, ogb_map_stats *stats)
+{
+	if (!c) { ogb_set_error("ogb_graph_map_reads: NULL context"); return OGB_E_ARG; }
+	if (!c->have_spelled) { ogb_set_error("ogb_graph_map_reads: run ogb_graph_spell on the uploaded reads first"); return OGB_E_STATE; }
+	const u64 nu = c->spst.unitigs, nw = c->spst.words, nb = 32 * nw + 1;
+	if (nb >= (1ull << 32)) { ogb_set_error("ogb_graph_map_reads: %llu bases of layout exceed the 32-bit positions", (unsigned long long)nb); return OGB_E_CAPACITY; }
+	if (n && (!bases || !offsets)) { ogb_set_error("ogb_graph_map_reads: NULL reads"); return OGB_E_ARG; }
+	for (u64 i = 0; i < n; i++)
+		if (offsets[i + 1] < offsets[i]) { ogb_set_error("ogb_graph_map_reads: offsets decrease at read %llu", (unsigned long long)i); return OGB_E_ARG; }
+	CUDA_TRY(cudaSetDevice(c->device));
+	c->mp_have_profile = false;
+	const u32 m = c->h + 1;
+	ogb_map_stats st = {};
+	st.reads_in = n; st.sample = c->mp_n_samples;
+	const int grid_max = c->sm_count * 8;
+	auto grid = [&](u64 items) { return (unsigned)std::max<u64>(1, std::min<u64>((items + 255) / 256, (u64)grid_max)); };
+	OGB_TRY(c->mp_ctr.ensure(8)); OGB_TRY(c->mp_rec.ensure(std::max<u64>(nu, 1))); OGB_TRY(c->mp_diff.ensure(nb)); OGB_TRY(c->mp_scan.ensure(nb));
+	u64 *ctr = c->mp_ctr.p;                                                       // [0] mapped, [1] multi, [2] placements, [3..4] filter stat, [5] kept, [6] scan total
+	CUDA_TRY(cudaEventRecord(c->ev[EV_T0], c->stream));
+	// ---- index over the layout, once per spell
+	const bool build_index = !c->mp_have_index;
+	if (build_index) {
+		c->mp_K = std::min<u32>(32, m + 1);
+		c->mp_buckets = mp_buckets(c->spst.bases);
+		OGB_TRY(c->mp_cnt.ensure(c->mp_buckets)); OGB_TRY(c->mp_bstart.ensure(c->mp_buckets + 1)); OGB_TRY(c->mp_ent.ensure(std::max<u64>(c->spst.bases, 1)));
+		CUDA_TRY(cudaMemsetAsync(c->mp_cnt.p, 0, c->mp_buckets * sizeof(u32), c->stream));
+		MapArgs A = map_args(c);
+		if (nw) k_map_count<<<grid(nw), 256, 0, c->stream>>>(A, nw, c->mp_cnt.p);
+		OGB_TRY(exclusive_scan(c, c->mp_cnt.p, (u32)c->mp_buckets, c->mp_bstart.p, c->mp_bstart.p + c->mp_buckets, nullptr, nullptr));
+		CUDA_TRY(cudaMemsetAsync(c->mp_cnt.p, 0, c->mp_buckets * sizeof(u32), c->stream));      // now the fill cursors
+		if (nw) k_map_fill<<<grid(nw), 256, 0, c->stream>>>(A, nw, c->mp_cnt.p, c->mp_ent.p);
+		CUDA_TRY(cudaGetLastError());
+		CUDA_TRY(cudaMemcpyAsync(&c->mp_entries, c->mp_bstart.p + c->mp_buckets, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+		st.launches += nw ? 5 : 3;
+	}
+	CUDA_TRY(cudaEventRecord(c->ev[EV_MP0], c->stream));
+	CUDA_TRY(cudaMemsetAsync(ctr, 0, 8 * sizeof(u64), c->stream));
+	CUDA_TRY(cudaMemsetAsync(c->mp_diff.p, 0, nb * sizeof(u32), c->stream));     // the difference array until the scan
+	if (nu) { k_cov_init<<<grid(nu), 256, 0, c->stream>>>(c->sp_rec.p, c->s_out.p, nu, c->mp_rec.p, nullptr); st.launches++; }
+	CUDA_TRY(cudaStreamSynchronize(c->stream));
+	c->mp_have_index = true;
+	// ---- the sample, chunk by chunk
+	for (u64 c0 = 0; c0 < n;) {
+		u64 c1 = c0 + 1;
+		while (c1 < n && c1 - c0 < OGB_MAP_CHUNK_READS && offsets[c1 + 1] - offsets[c0] <= OGB_MAP_CHUNK_BYTES) c1++;
+		const u32 nc = (u32)(c1 - c0);
+		const u64 nbytes = offsets[c1] - offsets[c0];
+		std::vector<u64> rel(nc + 1);
+		for (u32 i = 0; i <= nc; i++) rel[i] = offsets[c0 + i] - offsets[c0];
+		OGB_TRY(c->mp_raw.ensure(nbytes + 1)); OGB_TRY(c->mp_roffs.ensure(nc + 1)); OGB_TRY(c->mp_good.ensure(nc)); OGB_TRY(c->mp_pos.ensure(nc));
+		OGB_TRY(c->mp_start.ensure(nc)); OGB_TRY(c->mp_len.ensure(nc)); OGB_TRY(c->mp_khits.ensure(nc)); OGB_TRY(c->mp_meta.ensure(nc + 1));
+		CUDA_TRY(cudaEventRecord(c->ev[EV_MP1], c->stream));
+		CUDA_TRY(cudaMemcpyAsync(c->mp_raw.p, bases + offsets[c0], nbytes, cudaMemcpyHostToDevice, c->stream));
+		CUDA_TRY(cudaMemcpyAsync(c->mp_roffs.p, rel.data(), (nc + 1) * sizeof(u64), cudaMemcpyHostToDevice, c->stream));
+		const u64 stat[2] = {~0ull, 0};
+		CUDA_TRY(cudaMemcpyAsync(ctr + 3, stat, sizeof stat, cudaMemcpyHostToDevice, c->stream));
+		k_ds_filter<<<(nc + 127) / 128, 128, 0, c->stream>>>(c->mp_raw.p, c->mp_roffs.p, nc, m, c->mp_good.p, ctr + 3);
+		OGB_TRY(exclusive_scan(c, c->mp_good.p, nc, c->mp_pos.p, ctr + 5));
+		u64 h[3];
+		CUDA_TRY(cudaMemcpyAsync(h, ctr + 3, 3 * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+		CUDA_TRY(cudaStreamSynchronize(c->stream));
+		const u32 kept = (u32)h[2], max_pw = kept ? ((u32)(h[1] + 63) >> 6) << 1 : 0;
+		st.filtered += nc - kept;
+		st.launches += 4;
+		if (kept) {
+			// the chunk's read store: 2 pw words per read <= 4 (nbytes / 64 + kept), + the words a strand's last extract may touch
+			OGB_TRY(c->mp_words.ensure(4 * (nbytes / 64 + kept) + 8));
+			k_ds_compact<<<(nc + 255) / 256, 256, 0, c->stream>>>(c->mp_good.p, c->mp_pos.p, c->mp_roffs.p, nc, c->mp_start.p, c->mp_len.p);
+			k_map_geom<<<grid(kept), 256, 0, c->stream>>>(c->mp_len.p, kept, c->mp_khits.p);                 // (khits: scratch until k_map_reads)
+			OGB_TRY(exclusive_scan(c, c->mp_khits.p, kept, c->mp_meta.p, c->mp_meta.p + kept));
+			k_map_meta<<<grid(kept), 256, 0, c->stream>>>(c->mp_len.p, kept, c->mp_meta.p);
+			k_pack_ascii<<<(unsigned)(((u64)kept * max_pw + 255) / 256), 256, 0, c->stream>>>(c->mp_raw.p, c->mp_start.p, c->mp_words.p, c->mp_meta.p, kept, 0, 0, max_pw);
+			st.launches += 7;
+		}
+		CUDA_TRY(cudaEventRecord(c->ev[EV_MP2], c->stream));
+		if (kept) {
+			k_map_reads<<<grid(kept), 256, 0, c->stream>>>(map_args(c), kept, c->mp_diff.p, c->mp_rec.p, c->mp_khits.p, ctr);
+			st.launches++;
+		}
+		if (hits) {
+			OGB_TRY(c->mp_hits.ensure(nc));
+			k_map_hits<<<grid(nc), 256, 0, c->stream>>>(c->mp_good.p, c->mp_pos.p, c->mp_khits.p, nc, c->mp_hits.p);
+			CUDA_TRY(cudaMemcpyAsync(hits + c0, c->mp_hits.p, (size_t)nc * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
+			st.launches++;
+		}
+		CUDA_TRY(cudaGetLastError());
+		CUDA_TRY(cudaEventRecord(c->ev[EV_MP3], c->stream));
+		CUDA_TRY(cudaStreamSynchronize(c->stream));
+		st.ms_upload += ev_ms(c, EV_MP1, EV_MP2); st.ms_map += ev_ms(c, EV_MP2, EV_MP3);
+		c0 = c1;
+	}
+	// ---- depth
+	CUDA_TRY(cudaEventRecord(c->ev[EV_MP4], c->stream));
+	if (nu) {
+		OGB_TRY(exclusive_scan(c, c->mp_diff.p, (u32)nb, c->mp_scan.p, ctr + 6, nullptr, nullptr));
+		k_cov_reduce<<<grid(nw), 256, 0, c->stream>>>(c->mp_scan.p, c->sp_wpos.p, nu, nw, c->mp_diff.p, c->mp_rec.p);
+		CUDA_TRY(cudaGetLastError());
+		st.launches += 4;
+	}
+	CUDA_TRY(cudaEventRecord(c->ev[EV_T1], c->stream));
+	const size_t old = c->mp_samples.size();
+	c->mp_samples.resize(old + nu);
+	if (nu) CUDA_TRY(cudaMemcpyAsync(c->mp_samples.data() + old, c->mp_rec.p, nu * sizeof(ogb_unitig_coverage), cudaMemcpyDeviceToHost, c->stream));
+	u64 h[3];
+	CUDA_TRY(cudaMemcpyAsync(h, ctr, 3 * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+	const cudaError_t e = cudaStreamSynchronize(c->stream);
+	if (e != cudaSuccess) { c->mp_samples.resize(old); CUDA_TRY(e); }
+	st.mapped = h[0]; st.multi = h[1]; st.placements = h[2];
+	st.index_entries = c->mp_entries; st.index_buckets = c->mp_buckets;
+	st.ms = ev_ms(c, EV_T0, EV_T1); st.ms_index = build_index ? ev_ms(c, EV_T0, EV_MP0) : 0.f; st.ms_reduce = ev_ms(c, EV_MP4, EV_T1);
+	c->mp_n_samples++;
+	c->mp_have_profile = true;
+	if (stats) *stats = st;
+	return OGB_OK;
+}
+
+extern "C" int ogb_graph_sample_coverage(ogb_context *c, uint32_t sample, ogb_unitig_coverage *recs, uint64_t rec_cap, uint32_t *depth, uint64_t depth_cap)
+{
+	if (!c) { ogb_set_error("ogb_graph_sample_coverage: NULL context"); return OGB_E_ARG; }
+	if (!c->have_spelled || !c->mp_n_samples) { ogb_set_error("ogb_graph_sample_coverage: no sample mapped since the last ogb_graph_spell"); return OGB_E_STATE; }
+	if (sample >= c->mp_n_samples) { ogb_set_error("ogb_graph_sample_coverage: sample %u of %u", sample, c->mp_n_samples); return OGB_E_ARG; }
+	if (depth && (sample + 1 != c->mp_n_samples || !c->mp_have_profile)) { ogb_set_error("ogb_graph_sample_coverage: the profile is kept for the last sample only"); return OGB_E_ARG; }
+	const u64 nu = c->spst.unitigs, nd = 32 * c->spst.words;
+	if ((nu && (!recs || rec_cap < nu)) || (depth && depth_cap < nd)) {
+		ogb_set_error("ogb_graph_sample_coverage: need room for %llu records and %llu depth entries", (unsigned long long)nu, (unsigned long long)nd);
+		return OGB_E_CAPACITY;
+	}
+	if (nu) memcpy(recs, c->mp_samples.data() + (size_t)sample * nu, nu * sizeof(ogb_unitig_coverage));
+	if (depth && nd) {
+		CUDA_TRY(cudaSetDevice(c->device));
+		CUDA_TRY(cudaMemcpyAsync(depth, c->mp_diff.p, nd * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
+		CUDA_TRY(cudaStreamSynchronize(c->stream));
+	}
+	return OGB_OK;
+}
+
+extern "C" int ogb_graph_write_depths(ogb_context *c, const char *path, const char *const *names)
+{
+	if (!c || !path) { ogb_set_error("ogb_graph_write_depths: NULL argument"); return OGB_E_ARG; }
+	if (!c->have_spelled || !c->mp_n_samples) { ogb_set_error("ogb_graph_write_depths: no sample mapped since the last ogb_graph_spell"); return OGB_E_STATE; }
+	const u32 ns = c->mp_n_samples;
+	std::vector<std::string> nm(ns);
+	for (u32 j = 0; j < ns; j++) {
+		if (!names) { nm[j] = "sample_" + std::to_string(j); continue; }
+		if (!names[j] || strpbrk(names[j], "\t\n\r")) { ogb_set_error("ogb_graph_write_depths: sample name %u is NULL or holds a tab or a newline", j); return OGB_E_ARG; }
+		nm[j] = names[j];
+	}
+	const u64 nu = c->spst.unitigs;
+	FILE *f = fopen(path, "wb");
+	if (!f) { ogb_set_error("ogb_graph_write_depths: cannot open %s for writing", path); return OGB_E_IO; }
+	fprintf(f, "contigName\tcontigLen\ttotalAvgDepth");
+	for (u32 j = 0; j < ns; j++) fprintf(f, "\t%s\t%s-var", nm[j].c_str(), nm[j].c_str());
+	fputc('\n', f);
+	std::vector<double> mean(ns), var(ns);
+	for (u64 r = 0; r < nu; r++) {
+		const double len = (double)c->mp_samples[r].length;
+		double total = 0;
+		for (u32 j = 0; j < ns; j++) {
+			const ogb_unitig_coverage &v = c->mp_samples[(size_t)j * nu + r];
+			mean[j] = (double)v.depth_sum / len;
+			var[j] = std::max(0.0, (double)v.depth_sq_sum / len - mean[j] * mean[j]);
+			total += mean[j];
+		}
+		fprintf(f, "unitig_%llu\t%llu\t%.4f", (unsigned long long)(c->sp_first + r), (unsigned long long)c->mp_samples[r].length, total);
+		for (u32 j = 0; j < ns; j++) fprintf(f, "\t%.4f\t%.4f", mean[j], var[j]);
+		fputc('\n', f);
+	}
+	if (ferror(f)) { fclose(f); ogb_set_error("ogb_graph_write_depths: write to %s failed", path); return OGB_E_IO; }
+	if (fclose(f) != 0) { ogb_set_error("ogb_graph_write_depths: closing %s failed", path); return OGB_E_IO; }
 	return OGB_OK;
 }
 

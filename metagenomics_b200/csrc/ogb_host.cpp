@@ -155,6 +155,14 @@ extern "C" int ogb_dataset_add_file(ogb_dataset *ds, const char *path)
 	return OGB_OK;
 }
 
+extern "C" int ogb_dataset_raw_reads(const ogb_dataset *ds, const char **bases, const uint64_t **offsets, uint64_t *n)
+{
+	if (!ds || !bases || !offsets || !n) { ogb_set_error("ogb_dataset_raw_reads: NULL argument"); return OGB_E_ARG; }
+	if (ds->finalized) { ogb_set_error("ogb_dataset_raw_reads: the data set is finalized; its raw reads are gone"); return OGB_E_STATE; }
+	*bases = ds->raw.data(); *offsets = ds->raw_offs.data(); *n = ds->raw_offs.size() - 1;
+	return OGB_OK;
+}
+
 int ogb_dataset_filter(ogb_dataset *ds, uint32_t min_overlap, std::vector<uint64_t> &idx)
 {
 	if (!ds) { ogb_set_error("ogb_dataset_finalize: NULL dataset"); return OGB_E_ARG; }

@@ -136,6 +136,35 @@ bool OverlapGraph::saveUnitigCoverageToFile(string fileName)
 	return true;
 }
 
+// Maps the reads of every sample file (FASTA or FASTQ, read by the Dataset's parser) onto the unitigs simplifyGraph() spelled
+// (spellInBuild) and writes their depths as one table in MetaBAT's layout, one column pair per sample named after the file's basename
+// (ogb_graph_write_depths). The device context stays: call it before saveUnitigsToFile, which releases it.
+bool OverlapGraph::saveSampleDepthsToFile(string fileName, const vector<string> &sampleFiles)
+{
+	if (!hashTable) throw OgbFailure(OGB_E_STATE, "saveSampleDepthsToFile: no unitigs on the device (set OverlapGraph::spellInBuild before the build)");
+	ogb_context *ctx = hashTable->getContext();
+	lastMapStats.assign(sampleFiles.size(), ogb_map_stats());
+	vector<string> names(sampleFiles.size());
+	vector<const char *> cnames(sampleFiles.size());
+	for (size_t j = 0; j < sampleFiles.size(); j++) {
+		ogb_dataset *ds = NULL;
+		ogbCheck(ogb_dataset_create(&ds), "OverlapGraph::saveSampleDepthsToFile");
+		const char *bases = NULL;
+		const uint64_t *offsets = NULL;
+		uint64_t n = 0;
+		int rc = ogb_dataset_add_file(ds, sampleFiles[j].c_str());
+		if (rc == OGB_OK) rc = ogb_dataset_raw_reads(ds, &bases, &offsets, &n);
+		if (rc == OGB_OK) rc = ogb_graph_map_reads(ctx, bases, offsets, n, NULL, &lastMapStats[j]);
+		ogb_dataset_destroy(ds);
+		ogbCheck(rc, "OverlapGraph::saveSampleDepthsToFile");
+		const size_t slash = sampleFiles[j].find_last_of('/');
+		names[j] = slash == string::npos ? sampleFiles[j] : sampleFiles[j].substr(slash + 1);
+		cnames[j] = names[j].c_str();
+	}
+	ogbCheck(ogb_graph_write_depths(ctx, fileName.c_str(), cnames.data()), "OverlapGraph::saveSampleDepthsToFile");
+	return true;
+}
+
 // The unitigs simplifyGraph() spelled (spellInBuild) as FASTA, decoded on the device; then the table and its context go, as at :210.
 bool OverlapGraph::saveUnitigsToFile(string fileName)
 {

@@ -42,6 +42,7 @@ class OverlapGraph
 		ogb_simplify_stats lastSimplifyStats;
 		ogb_spell_stats lastSpellStats;
 		ogb_coverage_stats lastCoverageStats;
+		vector<ogb_map_stats> lastMapStats;
 
 	public:
 		bool flowComputed;
@@ -67,6 +68,8 @@ class OverlapGraph
 		void sortEdges();
 		bool saveGraphToFile(string fileName);			// OverlapGraph.cpp:1219-1259: the reference's .unitig text format
 		bool saveUnitigCoverageToFile(string fileName);	// per-base read depth of the spelled unitigs as TSV (ogb_graph_coverage); before saveUnitigsToFile
+		bool saveSampleDepthsToFile(string fileName, const vector<string> &sampleFiles);	// every sample file mapped onto the spelled unitigs
+														// (ogb_graph_map_reads), the depth table in MetaBAT's layout (ogb_graph_write_depths); before saveUnitigsToFile
 		bool saveUnitigsToFile(string fileName);		// the unitigs spelled in the build as FASTA (ogb_graph_write_unitigs); frees the hash table
 		bool readGraphFromFile(string fileName);		// OverlapGraph.cpp:1267-1367 (resume path, main.cpp:36-42)
 		Edge *findEdge(UINT64 source, UINT64 destination);
@@ -76,6 +79,7 @@ class OverlapGraph
 		const ogb_simplify_stats &getSimplifyStats(void) const { return lastSimplifyStats; }
 		const ogb_spell_stats &getSpellStats(void) const { return lastSpellStats; }
 		const ogb_coverage_stats &getCoverageStats(void) const { return lastCoverageStats; }
+		const vector<ogb_map_stats> &getMapStats(void) const { return lastMapStats; }	// one per sample of saveSampleDepthsToFile
 };
 
 #endif

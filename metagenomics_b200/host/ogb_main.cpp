@@ -5,11 +5,14 @@
 // this program produces and is not part of this library.
 //
 //   ogb_overlap -l minOverlap [-se n files...] [-pe n files...] [-f prefix] [--dump file] [--unitigs file] [--coverage file]
+//               [--samples n files... --depths file]
 //
 // --dump writes the graph in the binary format the parity tests read, so one comparator reads
 // the output of the unmodified reference and of this program. --unitigs writes the sequences of the canonical unitigs of the
 // simplified graph as FASTA, spelled on the device (OverlapGraph::spellInBuild, saveUnitigsToFile). --coverage writes their per-base
-// read depth summary as TSV, contained reads included (saveUnitigCoverageToFile); the names join with the FASTA's.
+// read depth summary as TSV, contained reads included (saveUnitigCoverageToFile); the names join with the FASTA's. --samples with
+// --depths maps the reads of every sample file onto the unitigs and writes the contig x sample depth table binners take, in MetaBAT's
+// layout, one column pair per sample named after the file's basename (saveSampleDepthsToFile).
 #include "Common.h"
 #include "Dataset.h"
 #include "Edge.h"
@@ -80,9 +83,10 @@ static void dumpMates(const char *path, Dataset *dataSet)
 int main(int argc, char **argv)
 {
 	UINT64 minimumOverlapLength = 0;
-	vector<string> pairedEndFileNames, singleEndFileNames;
+	vector<string> pairedEndFileNames, singleEndFileNames, sampleFileNames;
 	string allFileName = "";
-	const char *dumpPath = NULL, *resavePath = NULL, *matesPath = NULL, *unitigsPath = NULL, *coveragePath = NULL;
+	const char *dumpPath = NULL, *resavePath = NULL, *matesPath = NULL, *unitigsPath = NULL, *coveragePath = NULL, *depthsPath = NULL;
+	bool haveSamples = false;
 	bool startFromUnitigGraph = false;
 	for (int i = 1; i < argc; i++) {
 		string a = argv[i];
@@ -97,8 +101,13 @@ int main(int argc, char **argv)
 		else if (a == "--mates" && i + 1 < argc) matesPath = argv[++i];
 		else if (a == "--unitigs" && i + 1 < argc) unitigsPath = argv[++i];
 		else if (a == "--coverage" && i + 1 < argc) coveragePath = argv[++i];
+		else if (a == "--samples" && i + 1 < argc) {
+			int count = atoi(argv[++i]);
+			for (int k = 0; k < count && i + 1 < argc; k++) sampleFileNames.push_back(argv[++i]);
+			haveSamples = true;
+		} else if (a == "--depths" && i + 1 < argc) depthsPath = argv[++i];
 		else {
-			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file] [--unitigs file] [--coverage file]" << endl;
+			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file] [--unitigs file] [--coverage file] [--samples n files... --depths file]" << endl;
 			return a == "-h" || a == "--help" ? 0 : 1;
 		}
 	}
@@ -112,6 +121,14 @@ int main(int argc, char **argv)
 	}
 	if (startFromUnitigGraph && coveragePath) {
 		cerr << "ogb_overlap: --coverage needs the build on the device; -s resumes from a .unitig file without one" << endl;
+		return 1;
+	}
+	if (haveSamples != (depthsPath != NULL) || (haveSamples && sampleFileNames.empty())) {
+		cerr << "ogb_overlap: --samples (at least one file) and --depths go together" << endl;
+		return 1;
+	}
+	if (startFromUnitigGraph && depthsPath) {
+		cerr << "ogb_overlap: --samples / --depths need the build on the device; -s resumes from a .unitig file without one" << endl;
 		return 1;
 	}
 	try {
@@ -131,7 +148,7 @@ int main(int argc, char **argv)
 			return 0;
 		}
 		if (dumpPath) OverlapGraph::simplifyInBuild = false;											// --dump wants the graph as it is at OverlapGraph.cpp:210
-		if (unitigsPath || coveragePath) OverlapGraph::spellInBuild = true;
+		if (unitigsPath || coveragePath || depthsPath) OverlapGraph::spellInBuild = true;
 		HashTable *hashTable = new HashTable();															// main.cpp:45
 		hashTable->insertDataset(dataSet, minimumOverlapLength);										// main.cpp:46
 		overlapGraph = new OverlapGraph(hashTable); //hashTable deleted by this function after building the graph (main.cpp:47)
@@ -154,6 +171,16 @@ int main(int argc, char **argv)
 			const ogb_coverage_stats &cv = overlapGraph->getCoverageStats();
 			cout << "coverage: " << cv.unitigs << " unitigs " << cv.bases << " bases " << cv.placements << " placements " << cv.contained_placements
 			     << " contained placements " << cv.unplaced << " unplaced, coverage device ms: " << cv.ms << " (" << coveragePath << ")" << endl;
+		}
+		if (depthsPath) {
+			overlapGraph->saveSampleDepthsToFile(depthsPath, sampleFileNames);
+			for (size_t j = 0; j < sampleFileNames.size(); j++) {
+				const ogb_map_stats &mp = overlapGraph->getMapStats()[j];
+				const size_t slash = sampleFileNames[j].find_last_of('/');
+				cout << "map: " << (slash == string::npos ? sampleFileNames[j] : sampleFileNames[j].substr(slash + 1)) << " reads " << mp.reads_in
+				     << " filtered " << mp.filtered << " mapped " << mp.mapped << " multi " << mp.multi << " placements " << mp.placements
+				     << ", map device ms: " << mp.ms << " (" << depthsPath << ")" << endl;
+			}
 		}
 		if (unitigsPath) {
 			overlapGraph->saveUnitigsToFile(unitigsPath);
