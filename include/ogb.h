@@ -391,8 +391,10 @@ typedef struct ogb_coverage_stats {
 } ogb_coverage_stats; /* 64 bytes */
 
 /* The coverage of the unitigs of the last ogb_graph_spell (the same range and selection). freq = the frequency of every uploaded
- * read by ID - 1 (n = the uploaded read count; anything else is OGB_E_ARG), copied to the device per call. No spell on the
- * current reads: OGB_E_STATE. The result stays on the device until the next upload, build, simplify or spell. Integers only:
+ * read by ID - 1 (n = the uploaded read count; anything else is OGB_E_ARG), copied to the device per call. The frequencies must
+ * sum to less than 2^32, as the depth is kept in 32 bits: a larger sum is OGB_E_ARG, and the error names it (a Dataset's
+ * frequencies sum to its kept raw reads, below 2^32). No spell on the current reads: OGB_E_STATE. A refused call leaves the
+ * previous result as it was. The result stays on the device until the next upload, build, simplify or spell. Integers only:
  * two runs give the same bits. */
 int ogb_graph_coverage(ogb_context *ctx, const uint32_t *freq, uint64_t n, ogb_coverage_stats *stats);
 /* Copies the records of the last ogb_graph_coverage (rec_cap >= unitigs) and, when depth is not NULL, the u32 profile in the

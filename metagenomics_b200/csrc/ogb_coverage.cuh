@@ -20,7 +20,7 @@
 //                  word-aligned layout (atomicAdd mod 2^32), for the read and for each contained read of it
 //   (scan)         one GLOBAL exclusive scan of the difference array: every +f/-f pair of a unitig lies in [start, start + length],
 //                  so each unitig's net sum is 0 before the next start and no segment resets are needed. The scan sums in u64;
-//                  its low 32 bits are the depth, which is < 2^32.
+//                  its low 32 bits are the depth, which is < 2^32 (ogb_graph_coverage refuses frequencies that sum to 2^32 or more).
 //   k_cov_reduce   warp per 32 words, lane per base: D[p] = low 32 bits of scan[p + 1] written as the u32 profile, and sum, sum of
 //                  squares, min and max per unitig over [start, start + length); padding bases are written (as 0) but not reduced
 //

@@ -2076,6 +2076,9 @@ extern "C" int ogb_graph_coverage(ogb_context *c, const uint32_t *freq, uint64_t
 	if (n != c->n || (n && !freq)) { ogb_set_error("ogb_graph_coverage: need the frequencies of the %u uploaded reads (got %llu)", c->n, (unsigned long long)(freq ? n : 0)); return OGB_E_ARG; }
 	const u64 nu = c->spst.unitigs, nw = c->spst.words, nb = 32 * nw + 1, ni = c->sst.n_items;
 	if (nb >= (1ull << 32)) { ogb_set_error("ogb_graph_coverage: %llu bases of layout exceed the 32-bit scan", (unsigned long long)nb); return OGB_E_CAPACITY; }
+	u64 fsum = 0;                                                                 // the depth is kept in 32 bits (ogb_coverage.cuh)
+	for (u64 i = 0; i < n; i++) fsum += freq[i];
+	if (fsum >= (1ull << 32)) { ogb_set_error("ogb_graph_coverage: the frequencies sum to %llu, not below 2^32", (unsigned long long)fsum); return OGB_E_ARG; }
 	CUDA_TRY(cudaSetDevice(c->device));
 	c->have_covered = false;
 	const u32 nr = c->n;
