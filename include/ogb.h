@@ -413,10 +413,21 @@ int ogb_graph_write_coverage(ogb_context *ctx, const char *path);
  * filter for the build's minOverlap m (length > m and < 65536, ACGT only in either case, no base count >= (UINT64)(len*.8)). A
  * placement of a kept read s of length L is (u, p) with bases [p, p + L) of unitig u equal to s or to its reverse complement; a
  * read equal to its own reverse complement is tested on one strand only. Every placement adds 1 to the depth on [p, p + L). Raw reads
- * count one by one, and a read with several placements counts at each. Reads with errors or clipped alignments do not map.
+ * count one by one, and a read with several placements counts at each. Reads with indels or clipped alignments do not map.
+ *
+ * Substitutions (ogb_graph_map_reads_approx): with d = max_mismatches (0 <= d <= OGB_MAP_MAX_MISMATCHES) and K = min(32, m + 1), the
+ * key length of the index, a kept read of length L is searched with d_r = min(d, floor(L / K) - 1) substitutions (pigeonhole needs
+ * d_r + 1 disjoint K-mers in the read). With m = 50 (K = 32): 100 bp reads at most 2, 150 bp reads at most 3, reads shorter than 2K
+ * exactly only. A candidate (u, p, strand) has bases [p, p + L) inside unitig u; its mismatch count H is the Hamming distance to the
+ * read (strand 0) or its reverse complement (strand 1). The read's best stratum b is the least H over the candidates of both strands;
+ * the read is mapped iff b <= d_r, and its placements are the distinct (u, p) with min(H_fw, H_rc) == b (a (u, p) reached on both
+ * strands counts once). Ties all count, as for exact reads. d = 0 is the exact definition above, bit for bit; raising d never removes
+ * a placement (a read mapped at b counts the same placements at every d >= b), so the depth at d2 >= d1 is >= that at d1 on every base.
  * -------------------------------------------------------------------------------------------- */
 
 #define OGB_MAP_FILTERED 0xFFFFFFFFu /* hits[i] of a read the filter dropped */
+#define OGB_MAP_UNPLACED 0xFF        /* mismatches[i] of a read that is filtered or not mapped */
+#define OGB_MAP_MAX_MISMATCHES 8     /* the largest max_mismatches of ogb_graph_map_reads_approx */
 
 typedef struct ogb_map_stats {
 	uint64_t reads_in;
@@ -445,6 +456,13 @@ typedef struct ogb_map_stats {
  * bases: OGB_E_CAPACITY; NULL buffers with n > 0 or offsets that decrease: OGB_E_ARG. Integers only: two runs give the same bits.
  * An upload, build, simplify or spell drops the index and the samples. The coverage of ogb_graph_coverage is left as it is. */
 int ogb_graph_map_reads(ogb_context *ctx, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t *hits, ogb_map_stats *stats);
+/* ogb_graph_map_reads with up to max_mismatches substitutions per read (the definition above); ogb_graph_map_reads is this call with
+ * (0, hits, NULL). mismatches (NULL or n entries): every read's best stratum b, OGB_MAP_UNPLACED for a read that is filtered or not
+ * mapped. hits and the counters of stats (mapped, multi, placements) count best-stratum placements. Samples mapped with different
+ * max_mismatches share the index and append to the same list. max_mismatches > OGB_MAP_MAX_MISMATCHES: OGB_E_ARG; otherwise the
+ * errors of ogb_graph_map_reads. */
+int ogb_graph_map_reads_approx(ogb_context *ctx, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t max_mismatches, uint32_t *hits,
+                               uint8_t *mismatches, ogb_map_stats *stats);
 /* Copies the records of sample `sample` (rec_cap >= unitigs) and, when depth is not NULL, its u32 profile in the spell's word-aligned
  * layout (depth_cap >= 32 * ogb_spell_stats.words) -- kept for the last sample only: depth must be NULL for any other. No samples:
  * OGB_E_STATE; a sample beyond the last, or depth for an earlier one: OGB_E_ARG; OGB_E_CAPACITY names the sizes needed. */

@@ -77,6 +77,8 @@ class MapStats(C.Structure):
 
 
 OGB_MAP_FILTERED = 0xFFFFFFFF
+OGB_MAP_UNPLACED = 0xFF
+OGB_MAP_MAX_MISMATCHES = 8
 
 # every symbol include/ogb.h declares: name -> (restype, argtypes)
 _u64p = C.POINTER(C.c_uint64)
@@ -132,6 +134,7 @@ PROTOTYPES = {
     "ogb_graph_unitig_coverage": (C.c_int, [_vp, _vp, C.c_uint64, _vp, C.c_uint64]),
     "ogb_graph_write_coverage": (C.c_int, [_vp, C.c_char_p]),
     "ogb_graph_map_reads": (C.c_int, [_vp, _vp, _vp, C.c_uint64, _vp, C.POINTER(MapStats)]),
+    "ogb_graph_map_reads_approx": (C.c_int, [_vp, _vp, _vp, C.c_uint64, C.c_uint32, _vp, _vp, C.POINTER(MapStats)]),
     "ogb_graph_sample_coverage": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint64, _vp, C.c_uint64]),
     "ogb_graph_write_depths": (C.c_int, [_vp, C.c_char_p, _vp]),
     "ogb_get_stats": (C.c_int, [_vp, C.POINTER(Stats)]),

@@ -55,6 +55,24 @@ OGB_HD bool cv_equal(const cu64 *s, cu64 a, const cu64 *t, cu32 len)
 	return true;
 }
 
+// Hamming distance of s[a .. a + len) and t[0 .. len) on packed strands, 32 bases at a time; once it passes `limit` the count so far
+// (> limit) is returned
+OGB_HD cu32 cv_mismatches(const cu64 *s, cu64 a, const cu64 *t, cu32 len, cu32 limit)
+{
+	cu32 h = 0;
+	for (cu32 k = 0; k < len; k += 32) {
+		const cu32 n = len - k < 32 ? len - k : 32;
+		const cu64 x = sp_extract32(s, a + k) ^ t[k >> 5];
+#if defined(__CUDA_ARCH__)
+		h += __popcll((x | x >> 1) & 0x5555555555555555ull & sp_top_bases(n));
+#else
+		h += __builtin_popcountll((x | x >> 1) & 0x5555555555555555ull & sp_top_bases(n));
+#endif
+		if (h > limit) return h;
+	}
+	return h;
+}
+
 // thread = read idx i with sup[i] != 0: q_x against its super read (OGB_CV_UNPLACED when neither strand occurs); *super_idx = its idx
 OGB_HD cu32 cv_locate(const CovArgs &A, cu32 i, cu32 &super_idx)
 {

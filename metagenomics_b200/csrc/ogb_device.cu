@@ -217,6 +217,7 @@ struct ogb_context {
 	Pool<u64> mp_bstart, mp_ent, mp_roffs, mp_pos, mp_start, mp_meta, mp_words, mp_scan, mp_ctr;
 	Pool<char> mp_raw;
 	Pool<unsigned short> mp_len;
+	Pool<unsigned char> mp_kstrat, mp_strat;        // best stratum per kept read / per raw read of a chunk
 	Pool<ogb_unitig_coverage> mp_rec;
 	bool mp_have_index = false;
 	u32 mp_K = 0;
@@ -404,7 +405,7 @@ extern "C" void ogb_context_destroy(ogb_context *c)
 	c->cv_cstart.release(); c->cv_ppos.release(); c->cv_scan.release(); c->cv_rec.release();
 	c->mp_cnt.release(); c->mp_good.release(); c->mp_khits.release(); c->mp_hits.release(); c->mp_diff.release(); c->mp_bstart.release(); c->mp_ent.release();
 	c->mp_roffs.release(); c->mp_pos.release(); c->mp_start.release(); c->mp_meta.release(); c->mp_words.release(); c->mp_scan.release(); c->mp_ctr.release();
-	c->mp_raw.release(); c->mp_len.release(); c->mp_rec.release();
+	c->mp_raw.release(); c->mp_len.release(); c->mp_rec.release(); c->mp_kstrat.release(); c->mp_strat.release();
 	if (c->d_ctr) cudaFree(c->d_ctr);
 	if (c->d_tot) cudaFree(c->d_tot);
 	if (c->d_cursor) cudaFree(c->d_cursor);
@@ -2196,7 +2197,14 @@ static MapArgs map_args(const ogb_context *c)
 
 extern "C" int ogb_graph_map_reads(ogb_context *c, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t *hits, ogb_map_stats *stats)
 {
+	return ogb_graph_map_reads_approx(c, bases, offsets, n, 0, hits, NULL, stats);
+}
+
+extern "C" int ogb_graph_map_reads_approx(ogb_context *c, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t max_mismatches, uint32_t *hits,
+                                          uint8_t *mismatches, ogb_map_stats *stats)
+{
 	if (!c) { ogb_set_error("ogb_graph_map_reads: NULL context"); return OGB_E_ARG; }
+	if (max_mismatches > OGB_MAP_MAX_MISMATCHES) { ogb_set_error("ogb_graph_map_reads: max_mismatches %u > %u", max_mismatches, (unsigned)OGB_MAP_MAX_MISMATCHES); return OGB_E_ARG; }
 	if (!c->have_spelled) { ogb_set_error("ogb_graph_map_reads: run ogb_graph_spell on the uploaded reads first"); return OGB_E_STATE; }
 	const u64 nu = c->spst.unitigs, nw = c->spst.words, nb = 32 * nw + 1;
 	if (nb >= (1ull << 32)) { ogb_set_error("ogb_graph_map_reads: %llu bases of layout exceed the 32-bit positions", (unsigned long long)nb); return OGB_E_CAPACITY; }
@@ -2269,14 +2277,20 @@ extern "C" int ogb_graph_map_reads(ogb_context *c, const char *bases, const uint
 			st.launches += 7;
 		}
 		CUDA_TRY(cudaEventRecord(c->ev[EV_MP2], c->stream));
+		if (mismatches) { OGB_TRY(c->mp_kstrat.ensure(nc)); OGB_TRY(c->mp_strat.ensure(nc)); }
 		if (kept) {
-			k_map_reads<<<grid(kept), 256, 0, c->stream>>>(map_args(c), kept, c->mp_diff.p, c->mp_rec.p, c->mp_khits.p, ctr);
+			MapArgs A = map_args(c);
+			A.d = max_mismatches;
+			(max_mismatches ? k_map_reads<false> : k_map_reads<true>)<<<grid(kept), 256, 0, c->stream>>>(A, kept, c->mp_diff.p, c->mp_rec.p, c->mp_khits.p,
+			                                                                                           mismatches ? c->mp_kstrat.p : nullptr, ctr);
 			st.launches++;
 		}
-		if (hits) {
-			OGB_TRY(c->mp_hits.ensure(nc));
-			k_map_hits<<<grid(nc), 256, 0, c->stream>>>(c->mp_good.p, c->mp_pos.p, c->mp_khits.p, nc, c->mp_hits.p);
-			CUDA_TRY(cudaMemcpyAsync(hits + c0, c->mp_hits.p, (size_t)nc * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
+		if (hits || mismatches) {
+			if (hits) OGB_TRY(c->mp_hits.ensure(nc));
+			k_map_hits<<<grid(nc), 256, 0, c->stream>>>(c->mp_good.p, c->mp_pos.p, c->mp_khits.p, c->mp_kstrat.p, nc, hits ? c->mp_hits.p : nullptr,
+			                                            mismatches ? c->mp_strat.p : nullptr);
+			if (hits) CUDA_TRY(cudaMemcpyAsync(hits + c0, c->mp_hits.p, (size_t)nc * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
+			if (mismatches) CUDA_TRY(cudaMemcpyAsync(mismatches + c0, c->mp_strat.p, nc, cudaMemcpyDeviceToHost, c->stream));
 			st.launches++;
 		}
 		CUDA_TRY(cudaGetLastError());

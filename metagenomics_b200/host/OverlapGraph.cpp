@@ -137,9 +137,9 @@ bool OverlapGraph::saveUnitigCoverageToFile(string fileName)
 }
 
 // Maps the reads of every sample file (FASTA or FASTQ, read by the Dataset's parser) onto the unitigs simplifyGraph() spelled
-// (spellInBuild) and writes their depths as one table in MetaBAT's layout, one column pair per sample named after the file's basename
+// (spellInBuild), with up to maxMismatches substitutions per read (0: exact occurrences only), and writes their depths as one table in MetaBAT's layout, one column pair per sample named after the file's basename
 // (ogb_graph_write_depths). The device context stays: call it before saveUnitigsToFile, which releases it.
-bool OverlapGraph::saveSampleDepthsToFile(string fileName, const vector<string> &sampleFiles)
+bool OverlapGraph::saveSampleDepthsToFile(string fileName, const vector<string> &sampleFiles, uint32_t maxMismatches)
 {
 	if (!hashTable) throw OgbFailure(OGB_E_STATE, "saveSampleDepthsToFile: no unitigs on the device (set OverlapGraph::spellInBuild before the build)");
 	ogb_context *ctx = hashTable->getContext();
@@ -154,7 +154,7 @@ bool OverlapGraph::saveSampleDepthsToFile(string fileName, const vector<string> 
 		uint64_t n = 0;
 		int rc = ogb_dataset_add_file(ds, sampleFiles[j].c_str());
 		if (rc == OGB_OK) rc = ogb_dataset_raw_reads(ds, &bases, &offsets, &n);
-		if (rc == OGB_OK) rc = ogb_graph_map_reads(ctx, bases, offsets, n, NULL, &lastMapStats[j]);
+		if (rc == OGB_OK) rc = ogb_graph_map_reads_approx(ctx, bases, offsets, n, maxMismatches, NULL, NULL, &lastMapStats[j]);
 		ogb_dataset_destroy(ds);
 		ogbCheck(rc, "OverlapGraph::saveSampleDepthsToFile");
 		const size_t slash = sampleFiles[j].find_last_of('/');

@@ -68,8 +68,9 @@ class OverlapGraph
 		void sortEdges();
 		bool saveGraphToFile(string fileName);			// OverlapGraph.cpp:1219-1259: the reference's .unitig text format
 		bool saveUnitigCoverageToFile(string fileName);	// per-base read depth of the spelled unitigs as TSV (ogb_graph_coverage); before saveUnitigsToFile
-		bool saveSampleDepthsToFile(string fileName, const vector<string> &sampleFiles);	// every sample file mapped onto the spelled unitigs
-														// (ogb_graph_map_reads), the depth table in MetaBAT's layout (ogb_graph_write_depths); before saveUnitigsToFile
+		bool saveSampleDepthsToFile(string fileName, const vector<string> &sampleFiles, uint32_t maxMismatches = 0);	// every sample file mapped onto the
+														// spelled unitigs with up to maxMismatches substitutions per read (ogb_graph_map_reads_approx), the depth
+														// table in MetaBAT's layout (ogb_graph_write_depths); before saveUnitigsToFile
 		bool saveUnitigsToFile(string fileName);		// the unitigs spelled in the build as FASTA (ogb_graph_write_unitigs); frees the hash table
 		bool readGraphFromFile(string fileName);		// OverlapGraph.cpp:1267-1367 (resume path, main.cpp:36-42)
 		Edge *findEdge(UINT64 source, UINT64 destination);

@@ -5,14 +5,15 @@
 // this program produces and is not part of this library.
 //
 //   ogb_overlap -l minOverlap [-se n files...] [-pe n files...] [-f prefix] [--dump file] [--unitigs file] [--coverage file]
-//               [--samples n files... --depths file]
+//               [--samples n files... --depths file [--mismatches d]]
 //
 // --dump writes the graph in the binary format the parity tests read, so one comparator reads
 // the output of the unmodified reference and of this program. --unitigs writes the sequences of the canonical unitigs of the
 // simplified graph as FASTA, spelled on the device (OverlapGraph::spellInBuild, saveUnitigsToFile). --coverage writes their per-base
 // read depth summary as TSV, contained reads included (saveUnitigCoverageToFile); the names join with the FASTA's. --samples with
 // --depths maps the reads of every sample file onto the unitigs and writes the contig x sample depth table binners take, in MetaBAT's
-// layout, one column pair per sample named after the file's basename (saveSampleDepthsToFile).
+// layout, one column pair per sample named after the file's basename (saveSampleDepthsToFile); --mismatches lets every read count
+// with up to d substitutions (at most floor(L / K) - 1 for a read of length L, K = min(32, minOverlap + 1)).
 #include "Common.h"
 #include "Dataset.h"
 #include "Edge.h"
@@ -87,6 +88,7 @@ int main(int argc, char **argv)
 	string allFileName = "";
 	const char *dumpPath = NULL, *resavePath = NULL, *matesPath = NULL, *unitigsPath = NULL, *coveragePath = NULL, *depthsPath = NULL;
 	bool haveSamples = false;
+	int maxMismatches = -1;																			// -1: no --mismatches
 	bool startFromUnitigGraph = false;
 	for (int i = 1; i < argc; i++) {
 		string a = argv[i];
@@ -106,8 +108,16 @@ int main(int argc, char **argv)
 			for (int k = 0; k < count && i + 1 < argc; k++) sampleFileNames.push_back(argv[++i]);
 			haveSamples = true;
 		} else if (a == "--depths" && i + 1 < argc) depthsPath = argv[++i];
-		else {
-			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file] [--unitigs file] [--coverage file] [--samples n files... --depths file]" << endl;
+		else if (a == "--mismatches" && i + 1 < argc) {
+			char *end = NULL;
+			const long d = strtol(argv[++i], &end, 10);
+			if (!*argv[i] || *end || d < 0 || d > OGB_MAP_MAX_MISMATCHES) {
+				cerr << "ogb_overlap: --mismatches takes 0 to " << OGB_MAP_MAX_MISMATCHES << ", not " << argv[i] << endl;
+				return 1;
+			}
+			maxMismatches = (int)d;
+		} else {
+			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file] [--unitigs file] [--coverage file] [--samples n files... --depths file [--mismatches d]]" << endl;
 			return a == "-h" || a == "--help" ? 0 : 1;
 		}
 	}
@@ -125,6 +135,10 @@ int main(int argc, char **argv)
 	}
 	if (haveSamples != (depthsPath != NULL) || (haveSamples && sampleFileNames.empty())) {
 		cerr << "ogb_overlap: --samples (at least one file) and --depths go together" << endl;
+		return 1;
+	}
+	if (maxMismatches >= 0 && (!haveSamples || startFromUnitigGraph)) {
+		cerr << "ogb_overlap: --mismatches needs --samples and --depths, on the build on the device (not with -s)" << endl;
 		return 1;
 	}
 	if (startFromUnitigGraph && depthsPath) {
@@ -173,7 +187,7 @@ int main(int argc, char **argv)
 			     << " contained placements " << cv.unplaced << " unplaced, coverage device ms: " << cv.ms << " (" << coveragePath << ")" << endl;
 		}
 		if (depthsPath) {
-			overlapGraph->saveSampleDepthsToFile(depthsPath, sampleFileNames);
+			overlapGraph->saveSampleDepthsToFile(depthsPath, sampleFileNames, maxMismatches > 0 ? (uint32_t)maxMismatches : 0);
 			for (size_t j = 0; j < sampleFileNames.size(); j++) {
 				const ogb_map_stats &mp = overlapGraph->getMapStats()[j];
 				const size_t slash = sampleFileNames[j].find_last_of('/');

@@ -30,6 +30,28 @@ def sample_reads(seed, genomes, n_reads, len_min, len_max=None, weights=None, pa
     return bases[:int(offs[-1])], offs
 
 
+def substitute(seed, bases, rate):
+    """Sequencing substitutions: every base of the flat ASCII `bases` (upper-case ACGT) is replaced, independently with probability
+    `rate`, by one of the other three bases, uniformly. Returns a new array (bases itself when rate is 0)."""
+    if rate <= 0 or len(bases) == 0:
+        return bases
+    rng = np.random.default_rng(seed)
+    n = len(bases)
+    gaps = []
+    total = 0
+    while total < n:                                              # a Bernoulli process as geometric gaps between substituted bases
+        g = rng.geometric(rate, int(n * rate * 1.05) + 64)
+        gaps.append(g)
+        total += int(g.sum())
+    pos = np.cumsum(np.concatenate(gaps)) - 1
+    pos = pos[pos < n]
+    code = np.full(256, 0, np.uint8)
+    code[np.frombuffer(b"ACGT", np.uint8)] = np.arange(4, dtype=np.uint8)
+    out = np.array(bases, dtype=np.uint8, copy=True)
+    out[pos] = np.frombuffer(b"ACGT", np.uint8)[(code[out[pos]] + rng.integers(1, 4, len(pos), dtype=np.uint8)) % 4]
+    return out
+
+
 def _metagenome(seed, n_genomes, len_lo, len_hi, scale):
     rng = np.random.default_rng(seed)
     lens = (rng.uniform(len_lo, len_hi, n_genomes) * scale).astype(np.int64)
