@@ -178,6 +178,13 @@ int ogb_dataset_find_read(const ogb_dataset *ds, const char *bases, uint32_t len
  * sample files (ogb_dataset_add_file) for ogb_graph_map_reads. */
 int ogb_dataset_raw_reads(const ogb_dataset *ds, const char **bases, const uint64_t **offsets, uint64_t *n);
 
+/* Opt-in, before the first read is added (else OGB_E_STATE): ogb_dataset_add_file keeps each record's name -- its header after '>'
+ * or '@' up to the first space or tab, CR stripped -- and ogb_dataset_add_reads an empty one. Without it nothing is kept. */
+int ogb_dataset_keep_names(ogb_dataset *ds);
+/* The names kept so far, aligned with ogb_dataset_raw_reads: read i's name = (*chars)[(*offsets)[i] .. (*offsets)[i+1]). Views valid
+ * until the data set changes; for ogb_graph_map_reads_sam. No names kept, or a finalized data set: OGB_E_STATE. */
+int ogb_dataset_raw_names(const ogb_dataset *ds, const char **chars, const uint64_t **offsets);
+
 /* ----------------------------------------------------------------------------------------------
  * Device side.
  * -------------------------------------------------------------------------------------------- */
@@ -439,7 +446,7 @@ typedef struct ogb_map_stats {
 	uint64_t index_buckets;
 	uint32_t sample;          /* this sample's index among the samples mapped since the spell */
 	uint32_t launches;
-	float ms;                 /* device time of ogb_graph_map_reads = the four parts below */
+	float ms;                 /* device time of ogb_graph_map_reads = the four parts below (of ogb_graph_map_reads_sam: their sum) */
 	float ms_index;           /* index build; 0 when the index of an earlier sample was reused */
 	float ms_upload;          /* reads to the device, filter, packing */
 	float ms_map;             /* lookups, verification, difference array (and the hit counts to the host) */
@@ -474,6 +481,49 @@ int ogb_graph_sample_coverage(ogb_context *ctx, uint32_t sample, ogb_unitig_cove
  * trimming. names: one per sample (NULL: sample_<j>). No samples: OGB_E_STATE; a name with a tab or a newline: OGB_E_ARG; a file that
  * cannot be written: OGB_E_IO. */
 int ogb_graph_write_depths(ogb_context *ctx, const char *path, const char *const *names);
+
+/* SAM output of a sample (csrc/ogb_sam.cuh): the placements behind the depth, one alignment line per placement, readable by samtools,
+ * genome viewers and the binners that take alignments rather than a depth table. Single-end, unsorted, no BAM.
+ *
+ * Header, in this order: "@HD VN:1.6 SO:unsorted"; one "@SQ SN:unitig_<i> LN:<length>" per unitig of the last spell in record
+ * order (i as in ogb_graph_write_unitigs); "@PG ID:ogb_map PN:ogb CL:max_mismatches=<d>". Fields are separated by tabs.
+ * Records: every raw read, in input order, has at least one. With RNEXT *, PNEXT 0, TLEN 0 and QUAL * in every record:
+ *   dropped by the filter   1 record:  FLAG 4, RNAME *, POS 0, MAPQ 0, CIGAR *, SEQ = the raw bytes upper-cased with every non-letter
+ *                           written as N (* when empty), tag YF:Z:filtered
+ *   kept, not mapped        1 record:  FLAG 4, RNAME *, POS 0, MAPQ 0, CIGAR *, SEQ = the upper-case read
+ *   mapped, h placements    h records in ascending (u, p), the k-th (from 0) with FLAG 16 strand + 256 (k > 0), RNAME unitig_<i of u>,
+ *   in stratum b            POS p + 1, MAPQ 60 if h == 1 else 0, CIGAR <L>M, SEQ = the upper-case read, reverse-complemented on strand 1,
+ *                           tags NM:i:<b> MD:Z:<md> NH:i:<h>
+ * A placement (u, p) is on strand 0 iff the read itself (not its reverse complement) is within b substitutions there. MD is the SAM
+ * string of SEQ against bases [p, p + L) of the unitig: match counts and reference bases, starting and ending with a count, 0 between
+ * adjacent mismatches. MAPQ 60 / 0 is this project's convention for unique / multiple placements, not a probability.
+ * Every record adds 1 on [POS - 1, POS - 1 + L) of its unitig, so the pileup of the file is the sample's profile
+ * (ogb_graph_sample_coverage) on every base. Two runs write the same bytes. */
+typedef struct ogb_sam_stats {
+	uint64_t records;         /* lines after the header */
+	uint64_t bytes;           /* of the file, header included */
+	uint32_t launches;        /* of the SAM stages (the mapping's are in ogb_map_stats) */
+	/* Device times are sums of CUDA event intervals that enclose GPU work only (kernels, the copies of totals and of the text);
+	 * the host's waits for a total between them are left out, a launch's latency is not. */
+	float ms_emit;            /* device time: placement slots, the search again, the per-read sort */
+	float ms_format;          /* device time: record and byte offsets, slice cuts, the text */
+	float ms_copy;            /* device time: text to pinned host memory */
+	float ms_write;           /* host wall time in fwrite and fclose */
+	float ms_setup;           /* host wall time: name checks, the unitig records, opening the file, the header, and growing the two
+	                             pinned slice buffers (kept by the context, so only when a longer slice than before comes) */
+} ogb_sam_stats; /* 40 bytes */
+
+/* ogb_graph_map_reads_approx of one sample that also writes its SAM to `path`. Placements, hits, mismatches, the records, the profile
+ * and map_stats are bit for bit those of ogb_graph_map_reads_approx with the same arguments, and the sample is appended to the samples
+ * since the spell in the same way. QNAME: names == NULL and name_offsets == NULL: the read's 0-based index in the sample in decimal
+ * (the index of hits[i]); else read i's name is names[name_offsets[i] .. name_offsets[i+1]) and must match [!-?A-~]{1,254} (SAM's
+ * QNAME), or the call returns OGB_E_ARG naming the read before any work. Text is formatted on the device in slices and written by one
+ * host thread while the next slice is formatted; device memory does not grow with the sample. Errors: those of
+ * ogb_graph_map_reads_approx; a path that cannot be opened for writing is OGB_E_IO before any mapping, and a write that fails later is
+ * OGB_E_IO too. A refused or failed call leaves the list of samples as it was. */
+int ogb_graph_map_reads_sam(ogb_context *ctx, const char *bases, const uint64_t *offsets, uint64_t n, const char *names,
+                            const uint64_t *name_offsets, uint32_t max_mismatches, const char *path, uint32_t *hits, uint8_t *mismatches,
+                            ogb_map_stats *map_stats, ogb_sam_stats *sam_stats);
 
 int ogb_get_stats(ogb_context *ctx, ogb_stats *out);
 

@@ -76,6 +76,15 @@ class MapStats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_ if n != "reserved"}
 
 
+class SamStats(C.Structure):
+    """ogb_sam_stats (include/ogb.h)."""
+    _fields_ = [(n, C.c_uint64) for n in ("records", "bytes")] + [("launches", C.c_uint32)] + [
+        (n, C.c_float) for n in ("ms_emit", "ms_format", "ms_copy", "ms_write", "ms_setup")]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
 OGB_MAP_FILTERED = 0xFFFFFFFF
 OGB_MAP_UNPLACED = 0xFF
 OGB_MAP_MAX_MISMATCHES = 8
@@ -104,6 +113,8 @@ PROTOTYPES = {
     "ogb_dataset_get_read": (C.c_int, [_vp, C.c_uint64, C.c_int, _vp, C.c_uint32, C.POINTER(C.c_uint32)]),
     "ogb_dataset_find_read": (C.c_int, [_vp, C.c_char_p, C.c_uint32, _u64p]),
     "ogb_dataset_raw_reads": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_vp), _u64p]),
+    "ogb_dataset_keep_names": (C.c_int, [_vp]),
+    "ogb_dataset_raw_names": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_vp)]),
     "ogb_context_create": (C.c_int, [C.POINTER(_vp), C.c_int]),
     "ogb_nccl_unique_id": (C.c_int, [_vp]),
     "ogb_context_create_dist": (C.c_int, [C.POINTER(_vp), C.c_int, C.c_int, C.c_int, _vp]),
@@ -135,6 +146,8 @@ PROTOTYPES = {
     "ogb_graph_write_coverage": (C.c_int, [_vp, C.c_char_p]),
     "ogb_graph_map_reads": (C.c_int, [_vp, _vp, _vp, C.c_uint64, _vp, C.POINTER(MapStats)]),
     "ogb_graph_map_reads_approx": (C.c_int, [_vp, _vp, _vp, C.c_uint64, C.c_uint32, _vp, _vp, C.POINTER(MapStats)]),
+    "ogb_graph_map_reads_sam": (C.c_int, [_vp, _vp, _vp, C.c_uint64, _vp, _vp, C.c_uint32, C.c_char_p, _vp, _vp, C.POINTER(MapStats),
+                                          C.POINTER(SamStats)]),
     "ogb_graph_sample_coverage": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint64, _vp, C.c_uint64]),
     "ogb_graph_write_depths": (C.c_int, [_vp, C.c_char_p, _vp]),
     "ogb_get_stats": (C.c_int, [_vp, C.POINTER(Stats)]),

@@ -308,44 +308,68 @@ class OverlapGraph:
         check(lib().ogb_graph_write_coverage(self.ctx._h, str(path).encode()))
         return st
 
-    def map_reads(self, reads=None, bases=None, offsets=None, hits=False, max_mismatches=0, strata=False):
+    def map_reads(self, reads=None, bases=None, offsets=None, hits=False, max_mismatches=0, strata=False, sam=None, names=None):
         """Maps one sample -- a list of str/bytes reads, or flat ASCII bases + offsets (n + 1) -- onto the unitigs of the last spell()
         (ogb_graph_map_reads_approx): every read that passes the Dataset filter counts 1 on every placement of itself or its reverse
         complement with the fewest substitutions, at most min(max_mismatches, len // K - 1) (K = min(32, minOverlap + 1); 0: exact
         occurrences only). The sample is appended to the samples since that spell. Returns (records as COVERAGE_DTYPE in the unitig
         order: reads = read_count = placements, the ogb_map_stats as a dict[, hits][, strata]): hits = uint32 placements per read,
         OGB_MAP_FILTERED for a filtered read; strata = uint8 substitutions of each read's placements, OGB_MAP_UNPLACED for a read
-        that is filtered or not mapped."""
+        that is filtered or not mapped. sam: a path -- the placements are also written there as SAM (ogb_graph_map_reads_sam), and
+        the stats dict gains "sam" (the ogb_sam_stats); names (with sam only): one QNAME per read (str/bytes), else a read's QNAME is
+        its index."""
         if reads is not None:
             bases, offsets = _reads_to_buffers(reads)
         if bases is None:
             bases, offsets = np.zeros(0, np.uint8), np.zeros(1, np.uint64)
         bases = np.ascontiguousarray(bases, dtype=np.uint8)
         offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
-        return self._map(bases.ctypes.data, offsets.ctypes.data, len(offsets) - 1, hits, max_mismatches, strata)
+        nb = no = None
+        if names is not None:
+            if sam is None:
+                raise ValueError("names are the QNAMEs of a SAM: give sam= too")
+            if len(names) != len(offsets) - 1:
+                raise ValueError(f"{len(names)} names for {len(offsets) - 1} reads")
+            nb, no = _reads_to_buffers(names)                          # (kept referenced until the call returns)
+        return self._map(bases.ctypes.data, offsets.ctypes.data, len(offsets) - 1, hits, max_mismatches, strata, sam,
+                         None if nb is None else nb.ctypes.data, None if no is None else no.ctypes.data)
 
-    def map_file(self, path, hits=False, max_mismatches=0, strata=False):
-        """map_reads() of the reads of a FASTA or FASTQ file, read by the Dataset's parser (ogb_dataset_add_file)."""
+    def map_file(self, path, hits=False, max_mismatches=0, strata=False, sam=None):
+        """map_reads() of the reads of a FASTA or FASTQ file, read by the Dataset's parser (ogb_dataset_add_file); with sam, the
+        file's read names (its headers up to the first space or tab) are the QNAMEs."""
         ds = C.c_void_p()
         check(lib().ogb_dataset_create(C.byref(ds)))
         try:
+            if sam is not None:
+                check(lib().ogb_dataset_keep_names(ds))
             check(lib().ogb_dataset_add_file(ds, str(path).encode()))
             b, o, n = C.c_void_p(), C.c_void_p(), C.c_uint64()
             check(lib().ogb_dataset_raw_reads(ds, C.byref(b), C.byref(o), C.byref(n)))
-            return self._map(b.value, o.value, n.value, hits, max_mismatches, strata)
+            nb, no = C.c_void_p(), C.c_void_p()
+            if sam is not None:
+                check(lib().ogb_dataset_raw_names(ds, C.byref(nb), C.byref(no)))
+            return self._map(b.value, o.value, n.value, hits, max_mismatches, strata, sam, nb.value, no.value)
         finally:
             lib().ogb_dataset_destroy(ds)
 
-    def _map(self, bases, offsets, n, hits, max_mismatches=0, strata=False):
-        from ._lib import MapStats
+    def _map(self, bases, offsets, n, hits, max_mismatches=0, strata=False, sam=None, names=None, name_offsets=None):
+        from ._lib import MapStats, SamStats
         st = MapStats()
         h = np.zeros(n, np.uint32) if hits else None
         s = np.zeros(n, np.uint8) if strata else None
-        check(lib().ogb_graph_map_reads_approx(self.ctx._h, bases, offsets, n, int(max_mismatches), h.ctypes.data if hits else None,
-                                               s.ctypes.data if strata else None, C.byref(st)))
+        if sam is None:
+            check(lib().ogb_graph_map_reads_approx(self.ctx._h, bases, offsets, n, int(max_mismatches), h.ctypes.data if hits else None,
+                                                   s.ctypes.data if strata else None, C.byref(st)))
+        else:
+            ss = SamStats()
+            check(lib().ogb_graph_map_reads_sam(self.ctx._h, bases, offsets, n, names, name_offsets, int(max_mismatches), str(sam).encode(),
+                                                h.ctypes.data if hits else None, s.ctypes.data if strata else None, C.byref(st), C.byref(ss)))
         self._samples = st.sample + 1
         recs, _ = self.sample_depth(st.sample, profile=False)
-        return (recs, st.as_dict()) + ((h,) if hits else ()) + ((s,) if strata else ())
+        stats = st.as_dict()
+        if sam is not None:
+            stats["sam"] = ss.as_dict()
+        return (recs, stats) + ((h,) if hits else ()) + ((s,) if strata else ())
 
     def sample_depth(self, sample=-1, profile=True):
         """(records, profile) of a sample mapped since the last spell (-1: the last one): the profile is the uint32 per-base depth in

@@ -14,6 +14,7 @@
 #include "ogb_spell.cuh"
 #include "ogb_coverage.cuh"
 #include "ogb_map.cuh"
+#include "ogb_sam.cuh"
 
 #include <algorithm>
 #include <chrono>
@@ -225,6 +226,13 @@ struct ogb_context {
 	std::vector<ogb_unitig_coverage> mp_samples;   // spst.unitigs records per sample
 	u32 mp_n_samples = 0;
 	bool mp_have_profile = false;                    // mp_diff holds the profile of the last sample
+	// SAM of a sample (ogb_sam.cuh): per kept read its first slot, the sorted placements, per raw read its record count and first
+	// record, per record its line length and byte offset, the slice cuts, one slice of text, the chunk's read names
+	Pool<u32> sm_cnt, sm_len;
+	Pool<u64> sm_kslot, sm_slot, sm_rstart, sm_off, sm_cut, sm_noffs, sm_ctr;
+	Pool<char> sm_text, sm_names;
+	char *sm_stage[2] = {nullptr, nullptr};         // pinned host buffers of two text slices (grow-only, like the pools)
+	u64 sm_stage_cap = 0;
 	// L2 persistence window on the bucket summary (l2_keep_summary)
 	const void *l2_window_ptr = nullptr;
 	size_t l2_window_bytes = 0;
@@ -406,6 +414,9 @@ extern "C" void ogb_context_destroy(ogb_context *c)
 	c->mp_cnt.release(); c->mp_good.release(); c->mp_khits.release(); c->mp_hits.release(); c->mp_diff.release(); c->mp_bstart.release(); c->mp_ent.release();
 	c->mp_roffs.release(); c->mp_pos.release(); c->mp_start.release(); c->mp_meta.release(); c->mp_words.release(); c->mp_scan.release(); c->mp_ctr.release();
 	c->mp_raw.release(); c->mp_len.release(); c->mp_rec.release(); c->mp_kstrat.release(); c->mp_strat.release();
+	c->sm_cnt.release(); c->sm_len.release(); c->sm_kslot.release(); c->sm_slot.release(); c->sm_rstart.release(); c->sm_off.release();
+	c->sm_cut.release(); c->sm_noffs.release(); c->sm_ctr.release(); c->sm_text.release(); c->sm_names.release();
+	for (char *&p : c->sm_stage) { if (p) cudaFreeHost(p); p = nullptr; }
 	if (c->d_ctr) cudaFree(c->d_ctr);
 	if (c->d_tot) cudaFree(c->d_tot);
 	if (c->d_cursor) cudaFree(c->d_cursor);
@@ -2200,17 +2211,28 @@ extern "C" int ogb_graph_map_reads(ogb_context *c, const char *bases, const uint
 	return ogb_graph_map_reads_approx(c, bases, offsets, n, 0, hits, NULL, stats);
 }
 
-extern "C" int ogb_graph_map_reads_approx(ogb_context *c, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t max_mismatches, uint32_t *hits,
-                                          uint8_t *mismatches, ogb_map_stats *stats)
+// the refusals of every sample mapping, before any work
+static int map_check(ogb_context *c, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t max_mismatches)
 {
 	if (!c) { ogb_set_error("ogb_graph_map_reads: NULL context"); return OGB_E_ARG; }
 	if (max_mismatches > OGB_MAP_MAX_MISMATCHES) { ogb_set_error("ogb_graph_map_reads: max_mismatches %u > %u", max_mismatches, (unsigned)OGB_MAP_MAX_MISMATCHES); return OGB_E_ARG; }
 	if (!c->have_spelled) { ogb_set_error("ogb_graph_map_reads: run ogb_graph_spell on the uploaded reads first"); return OGB_E_STATE; }
-	const u64 nu = c->spst.unitigs, nw = c->spst.words, nb = 32 * nw + 1;
+	const u64 nb = 32 * c->spst.words + 1;
 	if (nb >= (1ull << 32)) { ogb_set_error("ogb_graph_map_reads: %llu bases of layout exceed the 32-bit positions", (unsigned long long)nb); return OGB_E_CAPACITY; }
 	if (n && (!bases || !offsets)) { ogb_set_error("ogb_graph_map_reads: NULL reads"); return OGB_E_ARG; }
 	for (u64 i = 0; i < n; i++)
 		if (offsets[i + 1] < offsets[i]) { ogb_set_error("ogb_graph_map_reads: offsets decrease at read %llu", (unsigned long long)i); return OGB_E_ARG; }
+	return OGB_OK;
+}
+
+struct SamSink;
+static int sam_chunk(ogb_context *c, SamSink &K, const MapArgs &A, u64 c0, u32 nc, u32 kept);
+
+// One sample, chunk by chunk (map_check passed). sam: NULL, or where each chunk's SAM records go after its mapping.
+static int map_sample(ogb_context *c, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t max_mismatches, uint32_t *hits,
+                      uint8_t *mismatches, ogb_map_stats *stats, SamSink *sam)
+{
+	const u64 nu = c->spst.unitigs, nw = c->spst.words, nb = 32 * nw + 1;
 	CUDA_TRY(cudaSetDevice(c->device));
 	c->mp_have_profile = false;
 	const u32 m = c->h + 1;
@@ -2277,12 +2299,13 @@ extern "C" int ogb_graph_map_reads_approx(ogb_context *c, const char *bases, con
 			st.launches += 7;
 		}
 		CUDA_TRY(cudaEventRecord(c->ev[EV_MP2], c->stream));
-		if (mismatches) { OGB_TRY(c->mp_kstrat.ensure(nc)); OGB_TRY(c->mp_strat.ensure(nc)); }
+		if (mismatches || sam) OGB_TRY(c->mp_kstrat.ensure(nc));
+		if (mismatches) OGB_TRY(c->mp_strat.ensure(nc));
 		if (kept) {
 			MapArgs A = map_args(c);
 			A.d = max_mismatches;
 			(max_mismatches ? k_map_reads<false> : k_map_reads<true>)<<<grid(kept), 256, 0, c->stream>>>(A, kept, c->mp_diff.p, c->mp_rec.p, c->mp_khits.p,
-			                                                                                           mismatches ? c->mp_kstrat.p : nullptr, ctr);
+			                                                                                           mismatches || sam ? c->mp_kstrat.p : nullptr, ctr);
 			st.launches++;
 		}
 		if (hits || mismatches) {
@@ -2297,6 +2320,11 @@ extern "C" int ogb_graph_map_reads_approx(ogb_context *c, const char *bases, con
 		CUDA_TRY(cudaEventRecord(c->ev[EV_MP3], c->stream));
 		CUDA_TRY(cudaStreamSynchronize(c->stream));
 		st.ms_upload += ev_ms(c, EV_MP1, EV_MP2); st.ms_map += ev_ms(c, EV_MP2, EV_MP3);
+		if (sam) {
+			MapArgs A = map_args(c);
+			A.d = max_mismatches;
+			OGB_TRY(sam_chunk(c, *sam, A, c0, nc, kept));
+		}
 		c0 = c1;
 	}
 	// ---- depth
@@ -2318,9 +2346,225 @@ extern "C" int ogb_graph_map_reads_approx(ogb_context *c, const char *bases, con
 	st.mapped = h[0]; st.multi = h[1]; st.placements = h[2];
 	st.index_entries = c->mp_entries; st.index_buckets = c->mp_buckets;
 	st.ms = ev_ms(c, EV_T0, EV_T1); st.ms_index = build_index ? ev_ms(c, EV_T0, EV_MP0) : 0.f; st.ms_reduce = ev_ms(c, EV_MP4, EV_T1);
+	if (sam) st.ms = st.ms_index + st.ms_upload + st.ms_map + st.ms_reduce;      // the events also span the SAM stages and the file writes
 	c->mp_n_samples++;
 	c->mp_have_profile = true;
 	if (stats) *stats = st;
+	return OGB_OK;
+}
+
+extern "C" int ogb_graph_map_reads_approx(ogb_context *c, const char *bases, const uint64_t *offsets, uint64_t n, uint32_t max_mismatches, uint32_t *hits,
+                                          uint8_t *mismatches, ogb_map_stats *stats)
+{
+	OGB_TRY(map_check(c, bases, offsets, n, max_mismatches));
+	return map_sample(c, bases, offsets, n, max_mismatches, hits, mismatches, stats, nullptr);
+}
+
+// ------------------------------------------------------------------------------------------------
+// SAM of a sample: see ogb_sam.cuh.
+// ------------------------------------------------------------------------------------------------
+// Bytes of text per slice: the device holds one slice at a time and the host two (pinned), so fwrite of one overlaps formatting of
+// the next. A slice is the records whose text starts in its 64 MB window; it ends with the last of them, so a record longer than
+// the window makes its slice longer (the buffers grow to the longest slice). The pinned buffers stay with the context.
+static const u64 OGB_SAM_SLICE = 64ull << 20;
+
+struct SamSink {
+	FILE *f = nullptr;
+	const char *path = nullptr;
+	const char *names = nullptr;                    // NULL: QNAME = the read's index
+	const uint64_t *name_offsets = nullptr;
+	// two pairs around spans of GPU work between host round trips; per stage buffer: write begin, write end, copy end
+	cudaEvent_t ev[10] = {};
+	ogb_sam_stats st = {};
+	double write_s = 0, setup_s = 0;
+	~SamSink()
+	{
+		for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e);
+	}
+};
+
+static double host_s(std::chrono::steady_clock::time_point t0) { return std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count(); }
+
+static float sam_ms(cudaEvent_t a, cudaEvent_t b)
+{
+	float ms = 0;
+	cudaEventElapsedTime(&ms, a, b);
+	return ms;
+}
+
+// the SAM records of chunk [c0, c0 + nc) (kept of them kept), after its k_map_reads and k_map_hits: slots, emit, record and byte
+// offsets, then slice by slice onto the file
+static int sam_chunk(ogb_context *c, SamSink &K, const MapArgs &A, u64 c0, u32 nc, u32 kept)
+{
+	const int grid_max = c->sm_count * 8;
+	auto grid = [&](u64 items) { return (unsigned)std::max<u64>(1, std::min<u64>((items + 255) / 256, (u64)grid_max)); };
+	OGB_TRY(c->sm_ctr.ensure(4)); OGB_TRY(c->sm_kslot.ensure((u64)kept + 1)); OGB_TRY(c->sm_cnt.ensure(nc)); OGB_TRY(c->sm_rstart.ensure((u64)nc + 1));
+	u64 *sctr = c->sm_ctr.p;
+	// ms_emit / ms_format add up event pairs that enclose GPU work only: the host's waits for a total, and what it does then, fall
+	// between the pairs
+	u64 P = 0;
+	if (kept) {
+		CUDA_TRY(cudaEventRecord(K.ev[0], c->stream));
+		OGB_TRY(exclusive_scan(c, c->mp_khits.p, kept, c->sm_kslot.p, sctr));
+		CUDA_TRY(cudaMemcpyAsync(&P, sctr, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+		CUDA_TRY(cudaEventRecord(K.ev[1], c->stream));
+		CUDA_TRY(cudaStreamSynchronize(c->stream));
+		K.st.ms_emit += sam_ms(K.ev[0], K.ev[1]);
+		K.st.launches += 3;
+	}
+	OGB_TRY(c->sm_slot.ensure(std::max<u64>(P, 1)));
+	CUDA_TRY(cudaEventRecord(K.ev[0], c->stream));
+	if (P) {
+		(A.d ? k_map_emit<false> : k_map_emit<true>)<<<grid(kept), 256, 0, c->stream>>>(A, kept, c->mp_khits.p, c->sm_kslot.p, c->sm_slot.p);
+		K.st.launches++;
+	}
+	CUDA_TRY(cudaEventRecord(K.ev[1], c->stream));
+	SamArgs S;
+	S.M = A; S.raw = c->mp_raw.p; S.roffs = c->mp_roffs.p; S.good = c->mp_good.p; S.pos = c->mp_pos.p; S.khits = c->mp_khits.p;
+	S.kstrat = c->mp_kstrat.p; S.kslot = c->sm_kslot.p; S.slot = c->sm_slot.p; S.rstart = c->sm_rstart.p; S.n = nc;
+	S.names = nullptr; S.noffs = nullptr; S.index0 = c0; S.first = c->sp_first;
+	std::vector<u64> rel;
+	if (K.names) {
+		const u64 a = K.name_offsets[c0], nbytes = K.name_offsets[c0 + nc] - a;
+		rel.resize((size_t)nc + 1);
+		for (u32 i = 0; i <= nc; i++) rel[i] = K.name_offsets[c0 + i] - a;
+		OGB_TRY(c->sm_names.ensure(nbytes + 1)); OGB_TRY(c->sm_noffs.ensure((u64)nc + 1));
+		CUDA_TRY(cudaMemcpyAsync(c->sm_names.p, K.names + a, nbytes, cudaMemcpyHostToDevice, c->stream));
+		CUDA_TRY(cudaMemcpyAsync(c->sm_noffs.p, rel.data(), ((size_t)nc + 1) * sizeof(u64), cudaMemcpyHostToDevice, c->stream));
+		S.names = c->sm_names.p; S.noffs = c->sm_noffs.p;
+	}
+	CUDA_TRY(cudaEventRecord(K.ev[2], c->stream));
+	k_sam_count<<<grid(nc), 256, 0, c->stream>>>(S, c->sm_cnt.p);
+	OGB_TRY(exclusive_scan(c, c->sm_cnt.p, nc, c->sm_rstart.p, c->sm_rstart.p + nc));
+	u64 R = 0;
+	CUDA_TRY(cudaMemcpyAsync(&R, c->sm_rstart.p + nc, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaEventRecord(K.ev[3], c->stream));
+	CUDA_TRY(cudaStreamSynchronize(c->stream));
+	K.st.ms_emit += sam_ms(K.ev[0], K.ev[1]);
+	K.st.ms_format += sam_ms(K.ev[2], K.ev[3]);
+	if (R >= (1ull << 32)) { ogb_set_error("ogb_graph_map_reads_sam: %llu records in one chunk exceed the 32-bit scan", (unsigned long long)R); return OGB_E_CAPACITY; }
+	OGB_TRY(c->sm_len.ensure(R)); OGB_TRY(c->sm_off.ensure(R + 1));
+	CUDA_TRY(cudaEventRecord(K.ev[0], c->stream));
+	k_sam_len<<<grid(R), 256, 0, c->stream>>>(S, R, c->sm_len.p);
+	OGB_TRY(exclusive_scan(c, c->sm_len.p, (u32)R, c->sm_off.p, c->sm_off.p + R));
+	u64 total = 0;
+	CUDA_TRY(cudaMemcpyAsync(&total, c->sm_off.p + R, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaEventRecord(K.ev[1], c->stream));
+	CUDA_TRY(cudaStreamSynchronize(c->stream));
+	K.st.ms_format += sam_ms(K.ev[0], K.ev[1]);
+	const u64 ns = (total + OGB_SAM_SLICE - 1) / OGB_SAM_SLICE;
+	OGB_TRY(c->sm_cut.ensure(2 * (ns + 1)));
+	CUDA_TRY(cudaEventRecord(K.ev[0], c->stream));
+	k_sam_cut<<<grid(ns + 1), 256, 0, c->stream>>>(c->sm_off.p, R, OGB_SAM_SLICE, ns, c->sm_cut.p, c->sm_cut.p + ns + 1);
+	std::vector<u64> cut(2 * (ns + 1));
+	CUDA_TRY(cudaMemcpyAsync(cut.data(), c->sm_cut.p, cut.size() * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaEventRecord(K.ev[1], c->stream));
+	CUDA_TRY(cudaStreamSynchronize(c->stream));
+	CUDA_TRY(cudaGetLastError());
+	K.st.launches += 9;
+	K.st.ms_format += sam_ms(K.ev[0], K.ev[1]);
+	// the slices: write s + 1 and its copy are queued before the host writes s to the file
+	std::vector<u64> sl;                                                           // non-empty slices: index s
+	u64 longest = 0;
+	for (u64 q = 0; q < ns; q++)
+		if (cut[q + 1] > cut[q]) { sl.push_back(q); longest = std::max(longest, cut[ns + 1 + q + 1] - cut[ns + 1 + q]); }
+	if (sl.empty()) return OGB_OK;
+	OGB_TRY(c->sm_text.ensure(longest));
+	if (c->sm_stage_cap < longest) {
+		const auto t0 = std::chrono::steady_clock::now();
+		for (char *&p : c->sm_stage) { if (p) cudaFreeHost(p); p = nullptr; }
+		c->sm_stage_cap = 0;
+		for (char *&p : c->sm_stage) CUDA_TRY(cudaMallocHost((void **)&p, longest));
+		c->sm_stage_cap = longest;
+		K.setup_s += host_s(t0);
+	}
+	auto queue = [&](size_t q) -> int {
+		const u64 s = sl[q], r0 = cut[s], r1 = cut[s + 1], bytes = cut[ns + 1 + s + 1] - cut[ns + 1 + s];
+		cudaEvent_t *e = K.ev + 4 + 3 * (q & 1);
+		CUDA_TRY(cudaEventRecord(e[0], c->stream));
+		k_sam_write<<<grid(r1 - r0), 256, 0, c->stream>>>(S, r0, r1, c->sm_off.p, c->sm_text.p);
+		CUDA_TRY(cudaGetLastError());
+		CUDA_TRY(cudaEventRecord(e[1], c->stream));
+		CUDA_TRY(cudaMemcpyAsync(c->sm_stage[q & 1], c->sm_text.p, bytes, cudaMemcpyDeviceToHost, c->stream));
+		CUDA_TRY(cudaEventRecord(e[2], c->stream));
+		K.st.launches++;
+		return OGB_OK;
+	};
+	OGB_TRY(queue(0));
+	for (size_t q = 0; q < sl.size(); q++) {
+		if (q + 1 < sl.size()) OGB_TRY(queue(q + 1));
+		cudaEvent_t *e = K.ev + 4 + 3 * (q & 1);
+		CUDA_TRY(cudaEventSynchronize(e[2]));
+		K.st.ms_format += sam_ms(e[0], e[1]);
+		K.st.ms_copy += sam_ms(e[1], e[2]);
+		const u64 s = sl[q], bytes = cut[ns + 1 + s + 1] - cut[ns + 1 + s];
+		const auto t0 = std::chrono::steady_clock::now();
+		const size_t wrote = fwrite(c->sm_stage[q & 1], 1, bytes, K.f);
+		K.write_s += host_s(t0);
+		if (wrote != bytes) { ogb_set_error("ogb_graph_map_reads_sam: write to %s failed", K.path); return OGB_E_IO; }
+	}
+	K.st.records += R;
+	K.st.bytes += total;
+	return OGB_OK;
+}
+
+extern "C" int ogb_graph_map_reads_sam(ogb_context *c, const char *bases, const uint64_t *offsets, uint64_t n, const char *names,
+                                       const uint64_t *name_offsets, uint32_t max_mismatches, const char *path, uint32_t *hits,
+                                       uint8_t *mismatches, ogb_map_stats *map_stats, ogb_sam_stats *sam_stats)
+{
+	const auto t_setup = std::chrono::steady_clock::now();
+	OGB_TRY(map_check(c, bases, offsets, n, max_mismatches));
+	if (!path) { ogb_set_error("ogb_graph_map_reads_sam: NULL path"); return OGB_E_ARG; }
+	if (n && !names != !name_offsets) { ogb_set_error("ogb_graph_map_reads_sam: names and name_offsets go together"); return OGB_E_ARG; }
+	if (n && names)
+		for (u64 i = 0; i < n; i++) {
+			const u64 a = name_offsets[i], b = name_offsets[i + 1];
+			bool ok = b > a && b - a <= 254;
+			for (u64 k = a; ok && k < b; k++) ok = names[k] >= '!' && names[k] <= '~' && names[k] != '@';
+			if (!ok) { ogb_set_error("ogb_graph_map_reads_sam: the name of read %llu is not a SAM QNAME ([!-?A-~]{1,254})", (unsigned long long)i); return OGB_E_ARG; }
+		}
+	CUDA_TRY(cudaSetDevice(c->device));
+	const u64 nu = c->spst.unitigs;
+	std::vector<ogb_unitig> rec(nu);
+	if (nu) {
+		CUDA_TRY(cudaMemcpyAsync(rec.data(), c->sp_rec.p, nu * sizeof(ogb_unitig), cudaMemcpyDeviceToHost, c->stream));
+		CUDA_TRY(cudaStreamSynchronize(c->stream));
+	}
+	SamSink K;
+	K.path = path;
+	K.names = n ? names : nullptr; K.name_offsets = name_offsets;
+	for (cudaEvent_t &e : K.ev) CUDA_TRY(cudaEventCreate(&e));
+	K.f = fopen(path, "wb");
+	if (!K.f) { ogb_set_error("ogb_graph_map_reads_sam: cannot open %s for writing", path); return OGB_E_IO; }
+	u64 header = 0;
+	int w = fprintf(K.f, "@HD\tVN:1.6\tSO:unsorted\n");
+	header += w > 0 ? (u64)w : 0;
+	for (u64 r = 0; r < nu; r++) {
+		w = fprintf(K.f, "@SQ\tSN:unitig_%llu\tLN:%llu\n", (unsigned long long)(c->sp_first + r), (unsigned long long)rec[r].length);
+		header += w > 0 ? (u64)w : 0;
+	}
+	w = fprintf(K.f, "@PG\tID:ogb_map\tPN:ogb\tCL:max_mismatches=%u\n", max_mismatches);
+	header += w > 0 ? (u64)w : 0;
+	K.setup_s += host_s(t_setup);
+	const size_t old = c->mp_samples.size();
+	int rc = map_sample(c, bases, offsets, n, max_mismatches, hits, mismatches, map_stats, &K);
+	cudaStreamSynchronize(c->stream);                                             // nothing may still copy into the stage buffers
+	const auto t0 = std::chrono::steady_clock::now();
+	const bool bad = ferror(K.f) != 0;
+	const bool closed = fclose(K.f) == 0;
+	K.write_s += host_s(t0);
+	if (rc == OGB_OK && (bad || !closed)) {
+		ogb_set_error("ogb_graph_map_reads_sam: %s %s failed", bad ? "write to" : "closing", path);
+		rc = OGB_E_IO;
+		c->mp_samples.resize(old);                                                // the sample is not kept without its SAM
+		c->mp_n_samples--;
+		c->mp_have_profile = false;
+	}
+	if (rc != OGB_OK) return rc;
+	K.st.bytes += header;
+	K.st.ms_write = (float)(K.write_s * 1e3);
+	K.st.ms_setup = (float)(K.setup_s * 1e3);
+	if (sam_stats) *sam_stats = K.st;
 	return OGB_OK;
 }
 

@@ -112,6 +112,7 @@ extern "C" int ogb_dataset_add_reads(ogb_dataset *ds, const char *bases, const u
 	for (uint64_t i = 1; i <= n; i++) {
 		if (offsets[i] < offsets[i - 1]) { ogb_set_error("ogb_dataset_add_reads: offsets not monotone at %llu", (unsigned long long)i); return OGB_E_ARG; }
 		ds->raw_offs.push_back(base + offsets[i] - first);
+		if (ds->keep_names) ds->name_offs.push_back(ds->names.size());   // no name
 	}
 	return OGB_OK;
 }
@@ -124,16 +125,25 @@ extern "C" int ogb_dataset_add_file(ogb_dataset *ds, const char *path)
 	if (!f) { ogb_set_error("Unable to open file: %s", path); return OGB_E_IO; }
 	std::string line;
 	if (!std::getline(f, line)) return OGB_OK;
+	auto chomp = [](std::string &s) { while (!s.empty() && (s.back() == '\r' || s.back() == '\n')) s.pop_back(); };
+	std::string name;                                                        // of the record being read: its header up to a space or tab
+	auto header = [&](std::string h) {                                      // any line may arrive here, an empty one too
+		if (!ds->keep_names) return;
+		chomp(h);
+		const size_t cut = h.size() > 1 ? h.find_first_of(" \t", 1) : std::string::npos;
+		name = h.size() > 1 ? h.substr(1, cut == std::string::npos ? std::string::npos : cut - 1) : std::string();
+	};
 	auto push = [&](const std::string &s) {
 		ds->raw.insert(ds->raw.end(), s.begin(), s.end());
 		ds->raw_offs.push_back(ds->raw.size());
+		if (ds->keep_names) { ds->names.insert(ds->names.end(), name.begin(), name.end()); ds->name_offs.push_back(ds->names.size()); }
 	};
-	auto chomp = [](std::string &s) { while (!s.empty() && (s.back() == '\r' || s.back() == '\n')) s.pop_back(); };
+	header(line);
 	if (line[0] == '>') {			// FASTA: header, then sequence lines up to the next '>'
 		std::string seq;
 		bool have = true;
 		while (std::getline(f, line)) {
-			if (!line.empty() && line[0] == '>') { push(seq); seq.clear(); have = true; continue; }
+			if (!line.empty() && line[0] == '>') { push(seq); seq.clear(); have = true; header(line); continue; }
 			chomp(line);
 			seq += line;
 		}
@@ -147,11 +157,28 @@ extern "C" int ogb_dataset_add_file(ogb_dataset *ds, const char *path)
 			chomp(seq);
 			push(seq);
 			if (!std::getline(f, line)) break;	// next '@' header
+			header(line);
 		}
 	} else {
 		ogb_set_error("Unknown input file format: %s", path);
 		return OGB_E_IO;
 	}
+	return OGB_OK;
+}
+
+extern "C" int ogb_dataset_keep_names(ogb_dataset *ds)
+{
+	if (!ds) { ogb_set_error("ogb_dataset_keep_names: NULL argument"); return OGB_E_ARG; }
+	if (ds->finalized || ds->raw_offs.size() > 1) { ogb_set_error("ogb_dataset_keep_names: call it before the first read is added"); return OGB_E_STATE; }
+	ds->keep_names = true;
+	return OGB_OK;
+}
+
+extern "C" int ogb_dataset_raw_names(const ogb_dataset *ds, const char **chars, const uint64_t **offsets)
+{
+	if (!ds || !chars || !offsets) { ogb_set_error("ogb_dataset_raw_names: NULL argument"); return OGB_E_ARG; }
+	if (!ds->keep_names || ds->finalized) { ogb_set_error("ogb_dataset_raw_names: the data set keeps no names (ogb_dataset_keep_names) or is finalized"); return OGB_E_STATE; }
+	*chars = ds->names.data(); *offsets = ds->name_offs.data();
 	return OGB_OK;
 }
 

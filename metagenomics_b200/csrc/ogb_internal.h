@@ -15,6 +15,9 @@ void ogb_set_error(const char *fmt, ...);
 struct ogb_dataset {
 	std::vector<char> raw;
 	std::vector<uint64_t> raw_offs{0};
+	bool keep_names = false;              // ogb_dataset_keep_names: the sample files' read names, aligned with raw_offs
+	std::vector<char> names;
+	std::vector<uint64_t> name_offs{0};
 	bool finalized = false;
 	uint32_t min_overlap = 0;
 	uint64_t n_good = 0, shortest = ~0ULL, longest = 0;

@@ -116,8 +116,10 @@ OGB_HD bool mp_walk(const MapArgs &A, const cu64 *t, cu32 j, cu32 L, VISIT visit
 // With d_r = 0, b = 0 and pass 2 is the exact lookup: seed 0 of each strand, cv_equal, no dedupe (H == 0 matches every seed) and no
 // strand test (H_fw(p) == H_rc(p) == 0 only for a palindrome, tested on one strand).
 // EXACT compiles the d = 0 body alone (k_map_reads<true>): the same work as before substitutions were searched.
-template <bool EXACT = false, class ADD, class PLACE>
-OGB_HD cu32 mp_read(const MapArgs &A, cu64 i, ADD add, PLACE place, cu32 &strat)
+// mp_search reports each placement as visit(p, u, L, strand): p the layout position, L the read's length, strand 0 iff H_fw(p) == b
+// (ogb_sam.cuh writes it); mp_read passes it to add (the difference array, as cv_place) and place(unitig).
+template <bool EXACT = false, class VISIT>
+OGB_HD cu32 mp_search(const MapArgs &A, cu64 i, VISIT visit, cu32 &strat)
 {
 	const cu64 m = A.rmeta[i];
 	const cu32 L = (cu32)(m & 0xFFFF), pw = ((L + 63) >> 6) << 1;
@@ -153,15 +155,22 @@ OGB_HD cu32 mp_read(const MapArgs &A, cu64 i, ADD add, PLACE place, cu32 &strat)
 					if (k != j) return true;
 					if (s && cv_mismatches(A.layout, p, fw, L, b) <= b) return true;
 				}
-				add(p, 1u);
-				add(p + L, 0xFFFFFFFFu);
-				place(u);
+				visit(p, u, L, s);
 				hits++;
 				return true;
 			});
 	}
 	strat = hits ? b : OGB_MAP_UNPLACED;
 	return hits;
+}
+template <bool EXACT = false, class ADD, class PLACE>
+OGB_HD cu32 mp_read(const MapArgs &A, cu64 i, ADD add, PLACE place, cu32 &strat)
+{
+	return mp_search<EXACT>(A, i, [&](cu64 p, cu64 u, cu32 L, int) {
+		add(p, 1u);
+		add(p + L, 0xFFFFFFFFu);
+		place(u);
+	}, strat);
 }
 template <class ADD, class PLACE>
 OGB_HD cu32 mp_read(const MapArgs &A, cu64 i, ADD add, PLACE place)

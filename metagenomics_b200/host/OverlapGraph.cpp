@@ -138,8 +138,9 @@ bool OverlapGraph::saveUnitigCoverageToFile(string fileName)
 
 // Maps the reads of every sample file (FASTA or FASTQ, read by the Dataset's parser) onto the unitigs simplifyGraph() spelled
 // (spellInBuild), with up to maxMismatches substitutions per read (0: exact occurrences only), and writes their depths as one table in MetaBAT's layout, one column pair per sample named after the file's basename
-// (ogb_graph_write_depths). The device context stays: call it before saveUnitigsToFile, which releases it.
-bool OverlapGraph::saveSampleDepthsToFile(string fileName, const vector<string> &sampleFiles, uint32_t maxMismatches)
+// (ogb_graph_write_depths). With samDir, each sample's placements go to samDir/<basename>.sam too, QNAME = the file's read names
+// (ogb_graph_map_reads_sam). The device context stays: call it before saveUnitigsToFile, which releases it.
+bool OverlapGraph::saveSampleDepthsToFile(string fileName, const vector<string> &sampleFiles, uint32_t maxMismatches, string samDir)
 {
 	if (!hashTable) throw OgbFailure(OGB_E_STATE, "saveSampleDepthsToFile: no unitigs on the device (set OverlapGraph::spellInBuild before the build)");
 	ogb_context *ctx = hashTable->getContext();
@@ -152,13 +153,21 @@ bool OverlapGraph::saveSampleDepthsToFile(string fileName, const vector<string> 
 		const char *bases = NULL;
 		const uint64_t *offsets = NULL;
 		uint64_t n = 0;
-		int rc = ogb_dataset_add_file(ds, sampleFiles[j].c_str());
-		if (rc == OGB_OK) rc = ogb_dataset_raw_reads(ds, &bases, &offsets, &n);
-		if (rc == OGB_OK) rc = ogb_graph_map_reads_approx(ctx, bases, offsets, n, maxMismatches, NULL, NULL, &lastMapStats[j]);
-		ogb_dataset_destroy(ds);
-		ogbCheck(rc, "OverlapGraph::saveSampleDepthsToFile");
 		const size_t slash = sampleFiles[j].find_last_of('/');
 		names[j] = slash == string::npos ? sampleFiles[j] : sampleFiles[j].substr(slash + 1);
+		const char *nm = NULL;
+		const uint64_t *noffs = NULL;
+		int rc = samDir.empty() ? OGB_OK : ogb_dataset_keep_names(ds);
+		if (rc == OGB_OK) rc = ogb_dataset_add_file(ds, sampleFiles[j].c_str());
+		if (rc == OGB_OK) rc = ogb_dataset_raw_reads(ds, &bases, &offsets, &n);
+		if (rc == OGB_OK && !samDir.empty()) rc = ogb_dataset_raw_names(ds, &nm, &noffs);
+		if (rc == OGB_OK) {
+			if (samDir.empty()) rc = ogb_graph_map_reads_approx(ctx, bases, offsets, n, maxMismatches, NULL, NULL, &lastMapStats[j]);
+			else rc = ogb_graph_map_reads_sam(ctx, bases, offsets, n, nm, noffs, maxMismatches, (samDir + "/" + names[j] + ".sam").c_str(), NULL, NULL,
+			                                  &lastMapStats[j], NULL);
+		}
+		ogb_dataset_destroy(ds);
+		ogbCheck(rc, "OverlapGraph::saveSampleDepthsToFile");
 		cnames[j] = names[j].c_str();
 	}
 	ogbCheck(ogb_graph_write_depths(ctx, fileName.c_str(), cnames.data()), "OverlapGraph::saveSampleDepthsToFile");

@@ -5,7 +5,7 @@
 // this program produces and is not part of this library.
 //
 //   ogb_overlap -l minOverlap [-se n files...] [-pe n files...] [-f prefix] [--dump file] [--unitigs file] [--coverage file]
-//               [--samples n files... --depths file [--mismatches d]]
+//               [--samples n files... --depths file [--mismatches d] [--sam dir]]
 //
 // --dump writes the graph in the binary format the parity tests read, so one comparator reads
 // the output of the unmodified reference and of this program. --unitigs writes the sequences of the canonical unitigs of the
@@ -13,14 +13,19 @@
 // read depth summary as TSV, contained reads included (saveUnitigCoverageToFile); the names join with the FASTA's. --samples with
 // --depths maps the reads of every sample file onto the unitigs and writes the contig x sample depth table binners take, in MetaBAT's
 // layout, one column pair per sample named after the file's basename (saveSampleDepthsToFile); --mismatches lets every read count
-// with up to d substitutions (at most floor(L / K) - 1 for a read of length L, K = min(32, minOverlap + 1)).
+// with up to d substitutions (at most floor(L / K) - 1 for a read of length L, K = min(32, minOverlap + 1)). --sam also writes the
+// placements of every sample's reads as SAM, dir/<basename of the sample file>.sam, with the file's read names (the directory is
+// created if missing).
 #include "Common.h"
 #include "Dataset.h"
 #include "Edge.h"
 #include "HashTable.h"
 #include "OverlapGraph.h"
 
+#include <cerrno>
 #include <cstring>
+#include <set>
+#include <sys/stat.h>
 
 static unsigned long long fnv1a(const string &s)
 {
@@ -86,7 +91,7 @@ int main(int argc, char **argv)
 	UINT64 minimumOverlapLength = 0;
 	vector<string> pairedEndFileNames, singleEndFileNames, sampleFileNames;
 	string allFileName = "";
-	const char *dumpPath = NULL, *resavePath = NULL, *matesPath = NULL, *unitigsPath = NULL, *coveragePath = NULL, *depthsPath = NULL;
+	const char *dumpPath = NULL, *resavePath = NULL, *matesPath = NULL, *unitigsPath = NULL, *coveragePath = NULL, *depthsPath = NULL, *samDir = NULL;
 	bool haveSamples = false;
 	int maxMismatches = -1;																			// -1: no --mismatches
 	bool startFromUnitigGraph = false;
@@ -108,6 +113,7 @@ int main(int argc, char **argv)
 			for (int k = 0; k < count && i + 1 < argc; k++) sampleFileNames.push_back(argv[++i]);
 			haveSamples = true;
 		} else if (a == "--depths" && i + 1 < argc) depthsPath = argv[++i];
+		else if (a == "--sam" && i + 1 < argc) samDir = argv[++i];
 		else if (a == "--mismatches" && i + 1 < argc) {
 			char *end = NULL;
 			const long d = strtol(argv[++i], &end, 10);
@@ -117,7 +123,7 @@ int main(int argc, char **argv)
 			}
 			maxMismatches = (int)d;
 		} else {
-			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file] [--unitigs file] [--coverage file] [--samples n files... --depths file [--mismatches d]]" << endl;
+			cerr << "Usage: ogb_overlap -l minOverlap [-pe n files...] [-se n files...] [-f prefix] [-s] [--dump file] [--resave file] [--unitigs file] [--coverage file] [--samples n files... --depths file [--mismatches d] [--sam dir]]" << endl;
 			return a == "-h" || a == "--help" ? 0 : 1;
 		}
 	}
@@ -140,6 +146,18 @@ int main(int argc, char **argv)
 	if (maxMismatches >= 0 && (!haveSamples || startFromUnitigGraph)) {
 		cerr << "ogb_overlap: --mismatches needs --samples and --depths, on the build on the device (not with -s)" << endl;
 		return 1;
+	}
+	if (samDir) {
+		set<string> seen;
+		bool clash = false;
+		for (size_t j = 0; j < sampleFileNames.size(); j++) {
+			const size_t slash = sampleFileNames[j].find_last_of('/');
+			clash |= !seen.insert(slash == string::npos ? sampleFileNames[j] : sampleFileNames[j].substr(slash + 1)).second;
+		}
+		if (!haveSamples || !depthsPath || startFromUnitigGraph || clash) {
+			cerr << "ogb_overlap: --sam needs --samples and --depths, on the build on the device (not with -s), and samples of distinct basenames" << endl;
+			return 1;
+		}
 	}
 	if (startFromUnitigGraph && depthsPath) {
 		cerr << "ogb_overlap: --samples / --depths need the build on the device; -s resumes from a .unitig file without one" << endl;
@@ -187,7 +205,8 @@ int main(int argc, char **argv)
 			     << " contained placements " << cv.unplaced << " unplaced, coverage device ms: " << cv.ms << " (" << coveragePath << ")" << endl;
 		}
 		if (depthsPath) {
-			overlapGraph->saveSampleDepthsToFile(depthsPath, sampleFileNames, maxMismatches > 0 ? (uint32_t)maxMismatches : 0);
+			if (samDir && mkdir(samDir, 0777) != 0 && errno != EEXIST) throw OgbFailure(OGB_E_IO, string("cannot create ") + samDir);
+			overlapGraph->saveSampleDepthsToFile(depthsPath, sampleFileNames, maxMismatches > 0 ? (uint32_t)maxMismatches : 0, samDir ? samDir : "");
 			for (size_t j = 0; j < sampleFileNames.size(); j++) {
 				const ogb_map_stats &mp = overlapGraph->getMapStats()[j];
 				const size_t slash = sampleFileNames[j].find_last_of('/');
